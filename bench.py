@@ -2,11 +2,16 @@
 """bench.py — BASELINE.json's metric: search nodes/sec (N-Queens all-solutions) and Sudoku
 puzzles/sec, on 1/2/4/8 B200, next to the reference dequan timed on the host cores.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...                      (N > 1, one rank per GPU, NCCL)
 
-One "step" = one complete solve of the workload through the C ABI.  The workload is the same at every N, so that the
-1/2/4/8-GPU series is a strong-scaling series of ONE job: BASELINE config C5, 17-Queens all-solutions (95 815 104
+--dump-outputs DIR: what the last HBM-resident step of each workload returned, as DIR/<name>.npy (float32 / float64):
+N-Queens {solutions, nodes} and first solution; for the batches, solution / node count / status of a fixed, seeded
+sample of the instances (`*_index` holds their indices) and the batch totals {sat, unsat, budget, nodes}.  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
+
+One "step" = one complete solve of the workload through the C ABI; every timed loop runs K of them.  The workload is
+the same at every N, so that the 1/2/4/8-GPU series is a strong-scaling series of ONE job: BASELINE config C5, 17-Queens all-solutions (95 815 104
 solutions / 5 474 619 051 nodes, tests/golden/reference_large.json; about 15 ms on one B200), FC-surviving prefixes
 dealt to the ranks by key, {solutions, nodes} summed with NCCL.  The line also carries `sudoku` (config C3, 1M puzzles,
 sharded over the ranks) and, at N == 1, `extra.nqueens14_1gpu` (config C2) and `extra.colouring` (config C4), each
@@ -173,6 +178,23 @@ def reference_arm(args):
     print(json.dumps(line), flush=True)
 
 
+def sample_rows(n, k):
+    """At most k of the n instance indices of a batch, ascending, chosen with a fixed seed: --dump-outputs writes the
+    per-instance outputs of these rows only, so that two runs with the same arguments dump the same rows."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_outputs(path, outputs):
+    """--dump-outputs: one float32 / float64 array per name as `path/<name>.npy`, at most 64 MB in all."""
+    assert all(a.dtype in (np.float32, np.float64) for a in outputs.values())
+    assert sum(a.nbytes for a in outputs.values()) <= 64_000_000
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def workload_config(n_gpus, n):
     return {"workload": f"nqueens{n}_count_all", "baseline_config": {17: "C5", 14: "C2"}.get(n, ""),
             "parallelism": "prefix split" + (f", keys dealt to {n_gpus} GPUs, NCCL sum" if n_gpus > 1 else ""),
@@ -193,7 +215,11 @@ def main():
     ap.add_argument("--no-sudoku", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each workload computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return reference_arm(args)
@@ -228,11 +254,11 @@ def main():
         model = api.Model(csp)
 
         def solve_step(m):
+            """-> (this rank's result, the whole job's result)"""
             loc = m.solve_tree("count", part_rank=rank, part_count=world, engine=args.engine)
             if world == 1:
-                return loc, loc.solutions, loc.nodes
-            g = multi.reduce_tree(loc, m.nodes_upto, "count", n, device=dev)
-            return loc, g.solutions, g.nodes
+                return loc, loc
+            return loc, multi.reduce_tree(loc, m.nodes_upto, "count", n, device=dev)
 
         def timed_steps(step_fn, k, w):
             tot, kern, launches = 0.0, 0.0, 0
@@ -240,11 +266,12 @@ def main():
                 flush.fill_(i & 0xFF)
                 sync_all()
                 t0 = time.perf_counter()
-                loc, sols, nodes = step_fn()
+                loc, res = step_fn()
                 # (at N > 1 the step ends with the all_gather of the ranks' records and its read-back: every rank holds
                 # the global answer here, so the step needs no second barrier; the MAX over ranks is taken below)
                 torch.cuda.synchronize()
                 dt = time.perf_counter() - t0
+                sols, nodes = res.solutions, res.nodes
                 assert (sols, nodes) == (want_sols, want_nodes), f"parity failure in bench step: {(sols, nodes)}"
                 if i >= w:
                     tot += dt
@@ -254,9 +281,9 @@ def main():
                 t = torch.tensor([tot, kern], dtype=torch.float64, device=dev)
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
                 tot, kern = float(t[0]), float(t[1])
-            return tot, kern, launches
+            return tot, kern, launches, res
 
-        tot, kern_ms, launches = timed_steps(lambda: solve_step(model), steps, warmup)
+        tot, kern_ms, launches, last = timed_steps(lambda: solve_step(model), steps, warmup)
         # roofline leg: the search kernel's own duration from CUDA events on its stream (DQ_TREE_TIME_KERNELS; the steps
         # above replay the solve as one CUDA graph, whose inner events cannot be read back); this rank's own node count
         dom_ms, dom_nodes, dom_records = 0.0, 0, 0
@@ -274,10 +301,12 @@ def main():
             r = solve_step(m)
             m.close()
             return r
-        e_tot, _, _ = timed_steps(e2e_step, steps, warmup)
+        e_tot, _, _, _ = timed_steps(e2e_step, steps, warmup)
         return {"n": n, "nodes": want_nodes, "steps": steps, "tot": tot, "kern_ms": kern_ms, "launches": launches, "e_tot": e_tot,
                 "dom_ms": dom_ms, "dom_nodes": dom_nodes, "dom_records": dom_records, "table_bytes": model.table_bytes(),
-                "engine": model.solve_tree("count", part_rank=rank, part_count=world, engine=args.engine).engine}
+                "engine": model.solve_tree("count", part_rank=rank, part_count=world, engine=args.engine).engine,
+                "outputs": {f"nqueens{n}": np.array([last.solutions, last.nodes], dtype=np.float64),
+                            f"nqueens{n}_first": np.array(last.first or [], dtype=np.float64)}}
 
     def queens_block(q, int_peak, hbm_peak, peak_src):
         n, steps = q["n"], q["steps"]
@@ -294,7 +323,7 @@ def main():
         sampler.start()
     n = 17
     Q = measure_queens(n, args.steps, args.warmup)
-    Q14 = measure_queens(14, max(args.steps, 10), args.warmup) if world == 1 and not args.no_extra else None
+    Q14 = measure_queens(14, args.steps, args.warmup) if world == 1 and not args.no_extra else None
     sudoku = None
     if not args.no_sudoku:
         sudoku = sudoku_section(args, torch, api, dev, world, rank, dist, flush)      # still inside the clock-sampling window
@@ -308,6 +337,12 @@ def main():
             dist.destroy_process_group()
         return
     clocks = sampler.stop()
+    if args.dump_outputs:
+        outputs = dict(Q["outputs"])
+        for part in (Q14["outputs"] if Q14 else {}, sudoku.pop("_outputs") if sudoku else {},
+                     colouring.pop("_outputs") if colouring else {}):
+            outputs.update(part)
+        dump_outputs(args.dump_outputs, outputs)
     int_peak, _ = api.measure_int_peak()
     hbm_peak, peak_src = peaks()
     qb = queens_block(Q, int_peak, hbm_peak, peak_src)
@@ -393,7 +428,7 @@ def sudoku_section(args, torch, api, dev, world=1, rank=0, dist=None, flush=None
     d_sol = torch.empty_like(d_cells)
     d_nodes = torch.empty(n, dtype=torch.int64, device=dev)
     d_status = torch.empty(n, dtype=torch.uint8, device=dev)
-    steps, warm = max(3, min(args.steps, 5)), 3
+    steps, warm = args.steps, 3
     kern, tot, launches, total_nodes = 0.0, 0.0, 0, 0
     for i in range(warm + steps):
         if flush is not None:
@@ -407,6 +442,15 @@ def sudoku_section(args, torch, api, dev, world=1, rank=0, dist=None, flush=None
         if i >= warm:
             tot += dt; kern += st.kernel_ms; launches += st.kernel_launches; total_nodes = st.total_nodes
     tot, kern = reduce_max(tot), reduce_max(kern)
+    dumped = None
+    if args.dump_outputs:           # the last HBM-resident step's outputs (at N > 1: this rank's shard)
+        rows = sample_rows(n, 65536)
+        idx = torch.from_numpy(rows).to(dev)
+        dumped = {"sudoku_index": (lo + rows).astype(np.float64),
+                  "sudoku_solution": d_sol[idx].cpu().numpy().astype(np.float32),
+                  "sudoku_nodes": d_nodes[idx].cpu().numpy().astype(np.float64),
+                  "sudoku_status": d_status[idx].cpu().numpy().astype(np.float32),
+                  "sudoku_totals": np.array([st.n_sat, st.n_unsat, st.n_budget, st.total_nodes], dtype=np.float64)}
     # host-buffer leg (pinned), copies inside the timed region
     h_cells = torch.from_numpy(cells).pin_memory()
     h_sol = torch.empty((n, 81), dtype=torch.uint8).pin_memory()
@@ -447,6 +491,8 @@ def sudoku_section(args, torch, api, dev, world=1, rank=0, dist=None, flush=None
            "e2e": {"value": n * steps / e_tot, "unit": "puzzles/s", "h2d_bytes_per_step": n * 81, "d2h_bytes_per_step": n * 90,
                    "ms_per_step": 1e3 * e_tot / steps},
            "gpu_launches": launches, "_kernel_pps": kpps}
+    if dumped is not None:
+        out["_outputs"] = dumped
     if not args.no_cpu and os.path.exists(REF_BIN):
         sample = min(n_shard, 16000)
         path = "/tmp/dq_bench_sudoku.txt"
@@ -469,7 +515,7 @@ def colouring_section(args, torch, api, dev, flush):
     from dequan_b200 import generators as G
     n, nv, k, c, budget = args.colouring_n, 200, 3, 4.2, 100_000
     off, edges = G.colouring_batch(n, nv, c)
-    steps, warm = 3, 3
+    steps, warm = args.steps, 3
     pad = (-2 * int(off[-1])) % 16
     d_edges = torch.from_numpy(np.concatenate([edges.reshape(-1), np.zeros(pad, dtype=np.uint8)])).to(dev)
     d_off = torch.from_numpy(off).to(dev)
@@ -489,6 +535,15 @@ def colouring_section(args, torch, api, dev, flush):
         if i >= warm:
             tot += dt; kern += st.kernel_ms; search += st.search_kernel_ms; launches += st.kernel_launches
     total_nodes = st.total_nodes
+    dumped = None
+    if args.dump_outputs:           # the last HBM-resident step's outputs
+        rows = sample_rows(n, 16384)
+        idx = torch.from_numpy(rows).to(dev)
+        dumped = {"colouring_index": rows.astype(np.float64),
+                  "colouring_colours": d_col[idx].cpu().numpy().astype(np.float32),
+                  "colouring_nodes": d_nodes[idx].cpu().numpy().astype(np.float64),
+                  "colouring_status": d_status[idx].cpu().numpy().astype(np.float32),
+                  "colouring_totals": np.array([st.n_sat, st.n_unsat, st.n_budget, st.total_nodes], dtype=np.float64)}
     h_edges = torch.from_numpy(edges.reshape(-1).copy()).pin_memory()
     h_col = torch.empty((n, nv), dtype=torch.uint8).pin_memory()
     h_nodes = torch.empty(n, dtype=torch.int64).pin_memory()
@@ -519,6 +574,8 @@ def colouring_section(args, torch, api, dev, flush):
                    "h2d_bytes_per_step": int(st2.h2d_bytes), "d2h_bytes_per_step": int(st2.d2h_bytes), "ms_per_step": 1e3 * e_tot / steps},
            "gpu_launches": launches, "engine": "lane per instance (k_graphs_adjacency x2, k_graphs_lane)",
            "_bytes_in": int(2 * off[-1] + 8 * (n + 1))}
+    if dumped is not None:
+        out["_outputs"] = dumped
     if not args.no_cpu and os.path.exists(REF_BIN):
         sample = min(n, 256)
         path = "/tmp/dq_bench_graphs.txt"
