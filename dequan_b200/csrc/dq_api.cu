@@ -397,12 +397,11 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
         else if (N <= 16) K = 7;                   // 14: 0.179 ms (depth 5: 0.172 with a bucket kernel twice as long: the step is
                                                    // bound by the first-solution warp either way); 15: 0.34 ms (depth 6 / 8: 0.40 /
                                                    // 0.38); 16: 1.51 ms (depth 8: 1.55)
-        else if (N == 17) K = 8;                   // 35 M records: 9.65 ms (depth 7 / 9: 9.68 / 10.24; the levels cost 0.16 / 0.44 / 1.44 ms)
-        else K = 8;
+        else K = 8;                                // 17: 35 M records, 9.65 ms (depth 7 / 9: 9.68 / 10.24; the levels cost 0.16 / 0.44 / 1.44 ms)
     }
     // (the bucket search reads no prefix keys from its records — its first-solution warp computes 64-bit keys, and the
     // partition deal happens at depth <= 5 — so the split may go deeper than 32-bit keys would allow)
-    // warps per CTA chosen so that the pools (buckets x 128 frames x 16 B + the staging buffer, per warp) pack an SM's shared memory best
+    // warps per CTA chosen so that the pools (buckets x 128 frames x 16 B per warp) pack an SM's shared memory best
     int bucket_warps = 4;
     // up to eight buckets (variables k+1 .. N-3; the records themselves stay in registers): the kernel compiled for exactly
     // that many; more: the general one (variables k .. N-3)
@@ -414,12 +413,13 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
                       k_queens_bucket_t<5, J>, k_queens_bucket_t<6, J>, k_queens_bucket_t<7, J>, k_queens_bucket_t<8, J>}
     static const BucketKernel kBucketKernels[2][9] = {DQ_QB_ROW(0), DQ_QB_ROW(5)};
 #undef DQ_QB_ROW
-    static const bool general_only = getenv("DQ_QUEENS_GENERAL") != nullptr;
+    // DQ_QUEENS_PLAIN_ROWS=1 (test hook): the plain-row kernels on every board, so that boards a test can count reach the
+    // kernels that boards of 23 and more queens get
     static const bool plain_rows = getenv("DQ_QUEENS_PLAIN_ROWS") != nullptr;
-    const bool compiled = N - 3 - K >= 1 && N - 3 - K <= 8 && !general_only;
+    const bool compiled = N - 3 - K >= 1 && N - 3 - K <= 8;
     const int n_buckets = compiled ? N - 3 - K : N - 2 - K;
     const BucketKernel bucket_kernel = compiled ? kBucketKernels[(N + 10 <= 32 && !plain_rows) ? 1 : 0][n_buckets] : k_queens_bucket;
-    const size_t per_warp = (size_t)n_buckets * kQueensBucketCap * sizeof(uint4) + kQueensStageBytes;
+    const size_t per_warp = (size_t)n_buckets * kQueensBucketCap * sizeof(uint4);
     {
         int best = 0;
         for (int w = 2; w <= kQueensBucketMaxWarps; w++) {
@@ -445,11 +445,10 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
     unsigned long long* ctrl = m->d_ctrl.p;     // [0]=cursor [1]=sols [2]=nodes [3]=best [8+l]=frontier size at depth l
     unsigned long long launches = 0, h_frontier_nodes = 0;
     float ms_total = 0, ms_search = 0;
-    const char* env_pl = getenv("DQ_QUEENS_PART_LEVEL");
-    const int part_level = std::min(K - 1, env_pl ? atoi(env_pl) : 4);     // measured: depth-5 keys balance 2/4/8 partitions within 3 %
+    constexpr int kQueensPartLevel = 4;                     // measured: depth-5 keys balance 2/4/8 partitions within 3 %
+    const int part_level = std::min(K - 1, kQueensPartLevel);
     // levels 0 .. head-1 in one single-CTA launch (a few hundred records at most, all above the partition level)
     const int head = std::max(0, std::min(std::min(K, part_level), 3));
-    static const bool use_graph = getenv("DQ_NO_GRAPH") == nullptr;
     for (int attempt = 0; attempt < 3; attempt++) {
         DQ_CUDA(m->q_records.reserve(cap));
         DQ_CUDA(m->q_records2.reserve(m->q_records.cap));
@@ -512,7 +511,7 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
         // per (model, split, partition, buffers) and replayed; anything that changes one of those re-captures it.
         bool queued = false;
         const bool time_kernels = (opts->flags & DQ_TREE_TIME_KERNELS) != 0;
-        if (use_graph && !time_kernels) {
+        if (!time_kernels) {
             const unsigned long long key[6] = {(unsigned long long)K | ((unsigned long long)opts->part_rank << 16) | ((unsigned long long)opts->part_count << 32),
                                                (unsigned long long)rcap, (unsigned long long)(uintptr_t)buf[0], (unsigned long long)(uintptr_t)buf[1],
                                                (unsigned long long)(uintptr_t)ctrl, (unsigned long long)(uintptr_t)m->q_first.p};
@@ -655,12 +654,8 @@ int dq_model_table_bytes(const dq_model* m, uint64_t* bytes) {
 
 }  // extern "C" (templates follow)
 
-// node budget of the root probe of dq_solve_tree (DQ_PROBE_NODES overrides it, 0 switches the probe off)
+// node budget of the root probe of dq_solve_tree
 constexpr unsigned long long kProbeNodes = 512;
-static unsigned long long env_ull(const char* name, unsigned long long dflt) {
-    const char* e = getenv(name);
-    return e ? strtoull(e, nullptr, 10) : dflt;
-}
 
 // enumeration request of dq_enumerate_solutions (null for a plain solve)
 struct EnumRequest {
@@ -702,8 +697,9 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
         if (rc != DQ_OK) return rc;
         if (occ_l < 1) lanes = false;
     }
-    // enough prefixes for 24 rounds of the resident warps — or, one subtree per lane, 6 rounds of the resident lanes
-    const long long want_prefixes = (lanes ? (long long)(occ_l * m->sm_count * kLaneTreeThreads * env_ull("DQ_LANE_TREE_ROUNDS", 1)) : resident_warps * 24) * opts->part_count;
+    // enough prefixes for 24 rounds of the resident warps — or, one subtree per lane, one round of the resident lanes
+    // (2 or 4 rounds are no faster: profiles/r2_generic_lane_tree.txt)
+    const long long want_prefixes = (lanes ? (long long)occ_l * m->sm_count * kLaneTreeThreads : resident_warps * 24) * opts->part_count;
 
     if (er) {
         DQ_CUDA(m->e_out.reserve(std::max<size_t>((size_t)er->cap * nv, 1)));
@@ -778,10 +774,9 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
     // Most ForwardCheckingStep calls of a modelling session are small (the reference's own scenarios take 88-193
     // nodes): one launch and one synchronisation answer them, instead of a synchronisation per frontier level.
     // Past the budget the probe's counts are dropped and the split search below starts over.
-    static const unsigned long long probe_nodes = env_ull("DQ_PROBE_NODES", kProbeNodes);
     bool probed = false;
-    if (probe_nodes && want_depth < 0 && opts->part_count == 1 && !er) {
-        rc = launch_dfs(0, 1, 0, 1, probe_nodes);
+    if (want_depth < 0 && opts->part_count == 1 && !er) {
+        rc = launch_dfs(0, 1, 0, 1, kProbeNodes);
         if (rc != DQ_OK) return rc;
         DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
         DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof h_ctrl, cudaMemcpyDeviceToHost, m->stream));
@@ -796,8 +791,7 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
 
     // ---- the forced head of the tree (one prefix per level) in one launch (k_expand_head) ----
     constexpr int kHeadCap = 1, kHeadMaxLevels = 96;
-    static const bool use_head = getenv("DQ_NO_HEAD") == nullptr;
-    if (!probed && use_head && max_depth > 0) {
+    if (!probed && max_depth > 0) {
         const int head_max = std::min(std::min(max_depth, kHeadMaxLevels), want_depth >= 0 ? want_depth : max_depth);
         // one slab: per level dmask, surv (W), child_off, parent_of (u32), node_off (u64), prefixes (cap x level bytes); then the table
         const size_t per_level = (size_t)kHeadCap * (2 * sizeof(W) + 4 + 4 + 8);
@@ -990,7 +984,7 @@ static int solve_tree_impl(dq_model* m, const dq_tree_opts* opts, dq_tree_result
     if (opts->engine == DQ_ENGINE_LANE && !count_all) {
         g_err = "the lane engines serve COUNT_ALL only"; return DQ_ERR_UNSUPPORTED;
     }
-    // DQ_NO_CLASS=1 (measurements, tests): no structural class engine, every model takes the generic path
+    // DQ_NO_CLASS=1 (test hook, also used for measurements): no structural class engine, every model takes the generic path
     static const bool no_class = getenv("DQ_NO_CLASS") != nullptr;
     m->last_queens_first = false;
     if (!no_class && !er && !count_all && m->cm.model_class == CLASS_QUEENS && m->cm.queens_n >= 3 && m->cm.queens_n <= kQueensMaxN &&
@@ -1277,28 +1271,10 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     A.status = status_dev; A.hard = m->s_hard.p; A.tasks = m->s_tasks.p; A.task_cap = task_cap;
     A.snaps = m->s_snaps.p; A.snap_cap = snap_cap; A.snap_state = m->s_snap_state.p; A.ctrl = ctrl; A.user_budget = opts ? opts->node_budget : 0;
     A.force_donate = opts && opts->task_nodes > 0 ? (unsigned)opts->task_nodes : 0u;
-    const char* env_dd = getenv("DQ_SUDOKU_DONATE_DEPTH");
-    A.donate_depth = env_dd ? atoi(env_dd) : 5;     // measured sweep: 1..12, flat optimum around 5
-    const char* env_dm = getenv("DQ_SUDOKU_DONATE_MIN");
-    const char* env_dg = getenv("DQ_SUDOKU_DONATE_GAP");
-    A.donate_min = env_dm ? (unsigned)atoi(env_dm) : kDonateMinNodes;
-    A.donate_gap = env_dg ? (unsigned)atoi(env_dg) : kDonateGap;
-    const char* env_sg = getenv("DQ_SUDOKU_SPLIT_GAP");
-    A.split_gap = env_sg ? (unsigned)atoi(env_sg) : kSplitGap;
-    const char* env_h = getenv("DQ_SUDOKU_HIDDEN_AFTER");
-    A.strong_hidden_after = env_h ? (unsigned)atoi(env_h) : kStrongHiddenAfter;
-    const char* env_q = getenv("DQ_SUDOKU_POP_QUORUM");
-    A.pop_quorum = env_q ? atoi(env_q) : kPopQuorum;
-    const char* env_fb = getenv("DQ_SUDOKU_FIRST_BUDGET");
-    A.first_budget = env_fb ? (unsigned)atoi(env_fb) : (n >= 400000 ? 3072u : 1024u);   // measured at 1 M: 1024 -> 32.7 ms, 2048 -> 30.3, 3072 -> 29.5; 125 k shards: flat 512-1024 (7.2 ms), 1536 -> 7.6
+    A.first_budget = n >= 400000 ? 3072u : 1024u;   // measured at 1 M: 1024 -> 32.7 ms, 2048 -> 30.3, 3072 -> 29.5; 125 k shards: flat 512-1024 (7.2 ms), 1536 -> 7.6
     if (A.force_donate) A.first_budget = std::min(A.first_budget, 4u * A.force_donate);       // tests: push work through the task path
-    const bool trace = getenv("DQ_TRACE") != nullptr;
-    cudaEvent_t ev[7] = {nullptr};
-    if (trace) for (auto& e : ev) cudaEventCreate(&e);
-    auto mark = [&](int i) { if (trace) cudaEventRecord(ev[i], m->stream); };
     const long long sms = m->sm_count;
     DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
-    mark(0);
     {
         int occ_d = 0;
         rc = max_ctas_per_sm(k_sudoku_digest, kDigestTile, kDigestSmem, &occ_d);
@@ -1307,15 +1283,13 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
         k_sudoku_digest<<<(unsigned)std::max<long long>(1, std::min<long long>(tiles, (long long)std::max(occ_d, 1) * sms)), kDigestTile, kDigestSmem, m->stream>>>(
             cells_dev, n, stride, m->s_digest.p, ctrl + SKC_MAX_BLANK);
     }
-    mark(1);
     // The lanes' stacks are sized for the instance with the most blanks (one 8-byte read-back after the digest, ~20 us):
     // with 30 givens that is 51 levels instead of 81, 354 bytes of shared memory per lane instead of 414, and a fifth CTA
     // (20 warps instead of 16) on every SM.
     unsigned long long* h_blank = m->pin + 117;
     DQ_CUDA(cudaMemcpyAsync(h_blank, ctrl + SKC_MAX_BLANK, sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
     DQ_CUDA(cudaStreamSynchronize(m->stream));
-    static const bool full_stack = getenv("DQ_SUDOKU_FULL_STACK") != nullptr;
-    const int levels = full_stack ? 81 : (int)std::min<unsigned long long>(std::max<unsigned long long>(*h_blank, 1), 81);
+    const int levels = (int)std::min<unsigned long long>(std::max<unsigned long long>(*h_blank, 1), 81);
     const size_t smem = offsetof(SudokuSmem, stk) + (size_t)levels * kSudokuBlock * sizeof(uint16_t);
     const size_t smem_strong = sudoku_strong_smem(levels);       // (30 givens: 36 KB per CTA, 24 warps per SM instead of 16)
     A.stack_levels = levels;
@@ -1328,10 +1302,8 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     if (occ_first < 1 || occ_count < 1 || occ_walk < 1 || occ_strong < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
     const long long ctas_first = std::max<long long>(1, std::min<long long>(occ_first * sms, (long long)((n + kSudokuBlock - 1) / kSudokuBlock)));
     k_sudoku_first<<<(unsigned)ctas_first, kSudokuBlock, smem, m->stream>>>(A);
-    mark(2);
     // the hard list's length stays on the device: the next three kernels are sized for the machine and find it in ctrl
     k_sudoku_strong<<<(unsigned)(occ_strong * sms), 128, smem_strong, m->stream>>>(A);
-    mark(3);
     // Host-buffer call without a node budget: every solution is final here (what follows only counts nodes), so the
     // 81 bytes per instance go home on the side stream while the counting stage runs.
     if (m->early_sol_host && !A.user_budget) {
@@ -1342,26 +1314,16 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
         m->early_sol_done = true;
     }
     k_sudoku_walk<<<(unsigned)std::min<long long>(occ_walk * sms, (long long)((n + kSudokuBlock - 1) / kSudokuBlock)), kSudokuBlock, smem, m->stream>>>(A);
-    mark(4);
     k_sudoku_count<<<(unsigned)(occ_count * sms), kSudokuBlock, smem, m->stream>>>(A);
-    mark(5);
     k_sudoku_finish<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(A, ctrl + SKC_TOTALS);
     DQ_CUDA(m->s_deferred.reserve(n));
     k_sudoku_collect_deferred<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(status_dev, n, m->s_deferred.p, ctrl + 10);
-    mark(6);
     unsigned long long launches = 7;
     DQ_CUDA(cudaGetLastError());
     unsigned long long hc[16];
     DQ_CUDA(cudaMemcpyAsync(hc, ctrl, sizeof hc, cudaMemcpyDeviceToHost, m->stream));
     DQ_CUDA(cudaStreamSynchronize(m->stream));
     m->s_tasks_used = std::min(hc[SKC_RESERVE], task_cap);
-    if (trace) {
-        float ms[6];
-        for (int i = 0; i < 6; i++) cudaEventElapsedTime(&ms[i], ev[i], ev[i + 1]);
-        fprintf(stderr, "[dq] sudoku: n=%lld hard=%llu tasks=%llu snaps=%llu err=%llu | ms digest %.3f first %.3f strong %.3f walk %.3f count %.3f finish %.3f\n",
-                (long long)n, hc[SKC_HARD], hc[SKC_RESERVE], hc[SKC_SNAP], hc[SKC_ERROR], ms[0], ms[1], ms[2], ms[3], ms[4], ms[5]);
-        for (auto& e : ev) cudaEventDestroy(e);
-    }
     if (hc[SKC_ERROR] & 2) { g_err = "sudoku task pool overflow"; return DQ_ERR_NOMEM; }
     if (hc[SKC_ERROR] || hc[SKC_OUTSTANDING]) {
         g_err = "internal: sudoku counting pipeline inconsistent (error bits " + std::to_string(hc[SKC_ERROR]) + ")";
@@ -1476,7 +1438,7 @@ static int run_graphs_lane(int nv, int k, const int64_t* edge_off, const GraphBa
     if (*h_over > 65535) { g_err = "an instance leaves more than 65535 edges outside its neighbour rows"; return DQ_ERR_UNSUPPORTED; }
     A.over_cap = (int)((*h_over + 1) & ~1ull);
     A.stride = graphs_record_bytes(A.nvp, A.rw, A.over_cap);
-    const bool packed = k <= 3 && getenv("DQ_GRAPHS_K4_LAYOUT") == nullptr;      // (byte 3 of the state words is free below four colours)
+    const bool packed = k <= 3;      // (byte 3 of the state words is free below four colours)
     // the overflow pairs a lane keeps in shared memory: as many as cost no CTA per SM (the rest are read from the record)
     A.over_smem = 0;
     {

@@ -248,7 +248,6 @@ __device__ __forceinline__ uint32_t shr_clamp(uint32_t x, uint32_t n) { uint32_t
 // queens_first_owned.  Bucket sizes live in registers, lane i holding the size of bucket i.
 constexpr int kQueensBucketMaxWarps = 12;             // warps per CTA: the host picks what packs an SM's shared memory best
 constexpr int kQueensBucketCap = 128;
-constexpr int kQueensStageBytes = 0;                  // (the pools fill an SM's shared memory to the byte at 17 queens: see the refill)
 
 // DFS-first solution of the part of the tree this partition owns, and the depth-k key of its prefix
 // (ForwardCheckingStep's own order, dequan.h:494-571).  Run by one warp in a kernel of its own, on a second stream
@@ -334,7 +333,7 @@ k_queens_bucket(QueensLaneArgs A) {
     const int N = A.n;
     const int L = N - 2 - A.k;                                   // buckets: depth k .. N-3 (frames of depth N-2 never reach a bucket: see below)
     const uint32_t hi = ~((1u << N) - 1u);
-    const uint32_t per_warp = (uint32_t)L * kQueensBucketCap * 16u + kQueensStageBytes;
+    const uint32_t per_warp = (uint32_t)L * kQueensBucketCap * 16u;
     const uint32_t bbase = (uint32_t)__cvta_generic_to_shared(qb_frames) + (uint32_t)wib * per_warp;
     uint32_t pf_n = 0;                                           // records prefetched into pf0 / pf1 (in flight or landed)
     uint4 pf0 = make_uint4(0u, 0u, 0u, 0u), pf1 = pf0;

@@ -112,12 +112,7 @@ struct SudokuArgs {
     unsigned long long* ctrl;              // control block, see SkCtrl
     unsigned long long user_budget;        // per-instance node budget of the API (0 = none)
     unsigned first_budget;                 // nodes k_sudoku_first spends on an instance before calling it hard
-    int donate_depth;                      // ... and only levels at least this far above the current one
-    unsigned donate_min, donate_gap;       // k_sudoku_count: a task gives a level away only when it is this old / this long after the last time
-    unsigned strong_hidden_after;          // k_sudoku_strong: value tries after which hidden-single propagation joins in
-    int pop_quorum;                        // extra step-back rounds run while at least this many lanes still stand on an exhausted level
     int stack_levels;                      // the most blanks any instance of the batch has: levels of the lanes' (and k_sudoku_strong's) stacks
-    unsigned split_gap;                    // k_sudoku_count: a task splits unasked every time it has counted this many nodes
     unsigned force_donate;                 // test knob: donate whenever a task is this many nodes old, hungry lanes or not (0 = off)
 };
 
@@ -562,7 +557,7 @@ k_sudoku_first(SudokuArgs A) {
         for (int rep = 0;; rep++) {
             const bool popping = L.have && !L.enter && L.passrem == 0;
             const uint32_t pm = __ballot_sync(0xFFFFFFFFu, popping);
-            if (pm == 0 || (rep > 0 && __popc(pm) < A.pop_quorum)) break;
+            if (pm == 0 || (rep > 0 && __popc(pm) < kPopQuorum)) break;
             if (popping && sk_pop(S, t, L)) {
                 // the whole tree is exhausted: ForwardCheckingStep returns false
                 A.nodes[L.puzzle] = (81 - L.nblank) + L.nodes_hi + L.nodes;
@@ -776,7 +771,7 @@ k_sudoku_strong(SudokuArgs A) {
                 if (lane == owner) D = (D & ~(0x3FFu << (10 * f))) | ((v | 0x200u) << (10 * f));
                 D &= ~(M.peer[p][lane] * v);
                 ++tries;
-                if (sk_propagate(D, M, lane, valid3, tries > A.strong_hidden_after, u0, u1, u2)) { ok = true; break; }
+                if (sk_propagate(D, M, lane, valid3, tries > kStrongHiddenAfter, u0, u1, u2)) { ok = true; break; }
             }
             __syncwarp();
             if (lane == 0) rest[l] = (uint16_t)d;
@@ -907,6 +902,7 @@ k_sudoku_walk(SudokuArgs A) {
 constexpr int kDonatePeriod = 32;
 constexpr uint32_t kDonateMinNodes = 48;    // a task younger than this keeps its stack to itself
 constexpr uint32_t kDonateGap = 96;         // ... and so does one that gave a level away fewer nodes ago than this
+constexpr int kDonateDepth = 5;             // ... and it gives away only levels at least this far above the current one (swept 1..12: flat optimum around 5)
 constexpr uint32_t kSplitGap = 512;         // a task splits unasked every time it has counted this many nodes (1 M puzzles, count stage: 4096 -> 11.0 ms, 1024 -> 10.2, 512 -> 9.9, 256 -> 10.0, 128 -> 33.8)
 
 __global__ void __launch_bounds__(kSudokuBlock)
@@ -996,8 +992,8 @@ k_sudoku_count(SudokuArgs A) {
             L.nodes = 0; L.nodes_hi = 0;
             L.passrem = 0; L.dom_rem = 0;
             L.have = true;
-            donate_at = A.force_donate ? A.force_donate : A.donate_min;
-            split_at = A.split_gap;
+            donate_at = A.force_donate ? A.force_donate : kDonateMinNodes;
+            split_at = kSplitGap;
             if (info & SKT_ROOT) {
                 // path values at the levels above, then the task's own value at its level: committed above
                 const int l0 = (int)(info & 0xFF);
@@ -1060,8 +1056,8 @@ k_sudoku_count(SudokuArgs A) {
                 if (want) {
                     int l = L.base_sp;
                     while (l < L.sp && (S.stk[l][t] & 0x1FF) == 0) ++l;
-                    if (l + A.donate_depth <= L.sp) hl = l;                               // a level close to the current one roots a tiny subtree
-                    else if (L.nodes >= split_at) split_at = L.nodes + A.split_gap / 4;     // nothing to give right now: look again soon
+                    if (l + kDonateDepth <= L.sp) hl = l;                               // a level close to the current one roots a tiny subtree
+                    else if (L.nodes >= split_at) split_at = L.nodes + kSplitGap / 4;     // nothing to give right now: look again soon
                 }
                 const uint32_t elig = __ballot_sync(0xFFFFFFFFu, hl >= 0);
                 const long long quota = min((long long)8, demand / (long long)total_warps + 1);
@@ -1070,7 +1066,7 @@ k_sudoku_count(SudokuArgs A) {
                     // read it); none free at this position: no piece this time, the task offers again a little later
                     const unsigned long long sslot = atomicAdd(A.ctrl + SKC_SNAP, 1ull) % A.snap_cap;
                     if (atomicCAS(A.snap_state + sslot, 0u, 1u) != 0u) {
-                        donate_at = L.nodes + A.donate_gap; split_at = L.nodes + A.split_gap / 4;
+                        donate_at = L.nodes + kDonateGap; split_at = L.nodes + kSplitGap / 4;
                     } else {
                         atomicAdd(A.ctrl + SKC_OUTSTANDING, 1ull);             // the piece exists from here on
                         const unsigned long long slot = atomicAdd(A.ctrl + SKC_RESERVE, 1ull);
@@ -1086,8 +1082,8 @@ k_sudoku_count(SudokuArgs A) {
                             __threadfence();
                             rec[2] = SKT_VALID | (uint32_t)L.base_sp | ((uint32_t)hl << 8);
                             L.base_sp = hl + 1;                                  // this task keeps the deeper levels
-                            donate_at = L.nodes + (A.force_donate ? A.force_donate : A.donate_gap);
-                            split_at = L.nodes + A.split_gap;
+                            donate_at = L.nodes + (A.force_donate ? A.force_donate : kDonateGap);
+                            split_at = L.nodes + kSplitGap;
                         }
                     }
                 }
@@ -1099,7 +1095,7 @@ k_sudoku_count(SudokuArgs A) {
         for (int rep = 0;; rep++) {
             const bool popping = L.have && !L.enter && L.passrem == 0;
             const uint32_t pm = __ballot_sync(0xFFFFFFFFu, popping);
-            if (pm == 0 || (rep > 0 && __popc(pm) < A.pop_quorum)) break;
+            if (pm == 0 || (rep > 0 && __popc(pm) < kPopQuorum)) break;
             if (popping && sk_pop(S, t, L)) {
                 atomicAdd(A.nodes + L.puzzle, L.nodes_hi + L.nodes);             // every node of the subtree is a node of the reference
                 L.have = false; closed = 1;
@@ -1117,7 +1113,7 @@ k_sudoku_count(SudokuArgs A) {
             sk_enter(S, t, L.c, bt, dom, pass);
             L.dom_rem = dom; L.passrem = pass; L.enter = false;
         }
-        if (L.nodes >= 0x80000000u) { L.nodes_hi += L.nodes; L.nodes = 0; donate_at = 0; split_at = A.split_gap; }
+        if (L.nodes >= 0x80000000u) { L.nodes_hi += L.nodes; L.nodes = 0; donate_at = 0; split_at = kSplitGap; }
 
         // ---------------- closed tasks leave the outstanding count ----------------
         {

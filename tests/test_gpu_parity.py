@@ -915,11 +915,10 @@ def test_generic_path_on_the_queens_class(golden, product_lib):
         assert line == f"{n} {g['solutions']} {g['nodes']} {g['first']} {want_engine}", line
 
 
-@pytest.mark.parametrize("var", ["DQ_QUEENS_PLAIN_ROWS", "DQ_QUEENS_GENERAL"])
+@pytest.mark.parametrize("var", ["DQ_QUEENS_PLAIN_ROWS"])
 def test_queens_bucket_kernel_variants(golden, product_lib, var):
     """The bucket kernels a 17-Queens solve does not pick: forward-check rows all in plain form (what boards of 23 and
-    more queens get) and the general kernel (bucket count at run time) on boards that normally get a compiled one.
-    The variables are read once per process, hence the subprocess."""
+    more queens get).  The variable is read once per process, hence the subprocess."""
     import subprocess
     import sys
     code = ("import sys; sys.path.insert(0, %r); from dequan_b200 import api; from dequan_b200.model import nqueens\n"
