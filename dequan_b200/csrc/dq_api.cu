@@ -10,6 +10,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "dequan_b200.h"
@@ -38,7 +39,8 @@ void set_last_error(const std::string& s) { g_err = s; }
 
 // Device memory comes from a per-thread cache of freed blocks: compiling and solving a fresh model per call (the
 // drop-in header's pattern: one CSP, one ForwardCheckingStep) must not pay cudaMalloc/cudaFree (each a device-wide
-// synchronisation) every time.  Blocks are handed back to the driver only by dq_trim() or at thread exit.
+// synchronisation) every time.  Blocks go back to the driver only through trim(): when more than 8 GiB are parked, when
+// cudaMalloc fails, and when a dq_solve_tree_multi worker ends.  At thread exit they are left to the driver.
 struct BlockCache {
     struct Block { void* p; size_t bytes; int dev; };
     std::vector<Block> free_blocks;
@@ -80,12 +82,19 @@ struct BlockCache {
 };
 static thread_local BlockCache g_cache;
 
+// A device block from the cache, handed back to it when the buffer is destroyed (or re-reserved).  A view does not own
+// what it points to.
 template <class T>
 struct DevBuf {
     T* p = nullptr;
     size_t cap = 0, bytes = 0;
     int dev = -1;                                        // the device the block lives on
     bool view = false;                                   // points into somebody else's block (never handed to the cache)
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap), bytes(o.bytes), dev(o.dev), view(o.view) { o.p = nullptr; o.cap = 0; o.bytes = 0; o.view = false; }
+    ~DevBuf() { release(); }
     void set_view(T* q, size_t n) { release(); p = q; cap = n; bytes = 0; view = true; }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
@@ -99,20 +108,43 @@ struct DevBuf {
     void release() { if (p && !view) g_cache.give(p, bytes, dev); p = nullptr; cap = 0; bytes = 0; view = false; }
 };
 
+// The pinned host words that queued copies read from and write to: a pageable target would cost a staging copy, and
+// an asynchronous copy into pageable memory holds the calling thread until it is done.  Each use has its own words.
+struct PinnedWords {
+    struct {                                   // solve_queens_first
+        unsigned long long key_nodes[2];       // best key, nodes
+        uint8_t solution[32];
+    } queens_first;
+    struct {                                   // solve_queens_lane: the captured CUDA graph copies to and from these
+        unsigned long long init[32];           // initial control block
+        uint4 root;                            // root record
+        unsigned long long ctrl[32];           // control block read back
+        uint8_t first[32];                     // first-solution bytes
+    } queens_lane;
+    unsigned long long level_totals[2];        // solve_tree_generic: children and nodes of one frontier level
+    unsigned long long head[38];               // k_expand_head's output, as far as it fits
+    unsigned long long sudoku_max_blank;       // run_batch_sudoku: most blanks of an instance
+    unsigned long long graphs_over;            // run_graphs_lane: longest overflow list
+    unsigned long long graphs_ctrl[8];         // run_batch_graphs: control block read back
+};
+static_assert(sizeof(PinnedWords) <= 1024, "the pinned control words outgrew 1 KB");
+
 // Stream + timing events are per thread and device, shared by every handle.
 struct DeviceCtx {
     int dev = -1, sm_count = 0;
     cudaStream_t stream = nullptr, stream2 = nullptr;          // stream2: side work that overlaps the main queue
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr, ev3 = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;          // ordering only (no timing)
-    unsigned long long* pin = nullptr;                         // 1 KB of pinned host memory: control words of the queued solves
+    PinnedWords* pin = nullptr;
 };
-static thread_local std::vector<DeviceCtx> g_ctx;
+// Never destroyed, like the streams, events and pinned words they hold: a handle keeps a pointer to the context of its
+// first solve, also after the thread that created the context has ended.
+static thread_local std::vector<DeviceCtx*> g_ctx;
 static cudaError_t device_ctx(DeviceCtx** out) {
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
-    for (DeviceCtx& c : g_ctx) if (c.dev == dev) { *out = &c; return cudaSuccess; }
+    for (DeviceCtx* c : g_ctx) if (c->dev == dev) { *out = c; return cudaSuccess; }
     DeviceCtx c;
     c.dev = dev;
     if ((e = cudaDeviceGetAttribute(&c.sm_count, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
@@ -124,11 +156,18 @@ static cudaError_t device_ctx(DeviceCtx** out) {
     if ((e = cudaStreamCreateWithFlags(&c.stream2, cudaStreamNonBlocking)) != cudaSuccess) return e;
     if ((e = cudaEventCreateWithFlags(&c.ev_fork, cudaEventDisableTiming)) != cudaSuccess) return e;
     if ((e = cudaEventCreateWithFlags(&c.ev_join, cudaEventDisableTiming)) != cudaSuccess) return e;
-    if ((e = cudaHostAlloc((void**)&c.pin, 1024, cudaHostAllocDefault)) != cudaSuccess) return e;
-    g_ctx.push_back(c);
-    *out = &g_ctx.back();
+    if ((e = cudaHostAlloc((void**)&c.pin, sizeof(PinnedWords), cudaHostAllocDefault)) != cudaSuccess) return e;
+    g_ctx.push_back(new DeviceCtx(c));
+    *out = g_ctx.back();
     return cudaSuccess;
 }
+
+// Waits for the stream when it goes out of scope.  Declared after a call's stack buffers, so that it runs before their
+// destructors: a block goes back to the cache only once the queue that uses it has drained.
+struct StreamDrain {
+    cudaStream_t s;
+    ~StreamDrain() { cudaStreamSynchronize(s); }
+};
 
 struct LevelArrays {               // kept per expansion level for FIRST-mode node accounting
     int n = 0;
@@ -136,6 +175,10 @@ struct LevelArrays {               // kept per expansion level for FIRST-mode no
     DevBuf<unsigned long long> dmask64, surv64;           // dmask / surv of models with 64-bit domain words
     DevBuf<unsigned long long> node_off;
     DevBuf<uint8_t> prefixes;      // [n][depth]
+    void release_views() {
+        auto drop = [](auto& b) { if (b.view) b.release(); };
+        drop(dmask); drop(surv); drop(child_off); drop(parent_of); drop(dmask64); drop(surv64); drop(node_off); drop(prefixes);
+    }
 };
 
 }  // namespace dq
@@ -147,15 +190,10 @@ static void multi_destroy(MultiCtx* mc);
 
 struct dq_model {
     CompiledModel cm;
-    bool uploaded = false;
-    int device = -1;                            // the CUDA device the handle was first solved on
-    cudaStream_t stream = nullptr, stream2 = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr, ev3 = nullptr, ev_fork = nullptr, ev_join = nullptr;
-    unsigned long long* pin = nullptr;          // pinned control words (DeviceCtx)
+    DeviceCtx* ctx = nullptr;                   // the device context of the first solve; null until the tables are uploaded
     // the queue of one N-Queens solve (copies, level kernels, search, first solution) as an instantiated CUDA graph
     cudaGraphExec_t q_exec = nullptr;
     unsigned long long q_exec_key[6] = {0, 0, 0, 0, 0, 0}, q_seen_key[6] = {0, 0, 0, 0, 0, 0};
-    int sm_count = 0;
     // model tables in HBM
     DevBuf<uint8_t> d_blob;                     // all tables, one block
     std::vector<uint8_t> h_blob;                // its host image (kept while the copy may be in flight)
@@ -201,6 +239,10 @@ struct dq_model {
     unsigned long long s_tasks_used = 0;
     // dq_solve_tree_multi: one worker thread + one clone of the compiled model per device
     struct MultiCtx* multi = nullptr;
+    ~dq_model() {
+        if (multi) multi_destroy(multi);
+        if (q_exec) cudaGraphExecDestroy(q_exec);
+    }
 };
 
 namespace dq {
@@ -208,17 +250,13 @@ namespace dq {
 static int upload(dq_model* m) {
     int dev = 0;
     DQ_CUDA(cudaGetDevice(&dev));
-    if (m->uploaded) {
+    if (m->ctx) {
         // a handle is bound to the device (and thread) of its first solve: its stream, events and cached blocks live there
-        if (dev != m->device) { g_err = "model handle is bound to CUDA device " + std::to_string(m->device) + " (dq_set_device before the first solve)"; return DQ_ERR_INVALID; }
+        if (dev != m->ctx->dev) { g_err = "model handle is bound to CUDA device " + std::to_string(m->ctx->dev) + " (dq_set_device before the first solve)"; return DQ_ERR_INVALID; }
         return DQ_OK;
     }
-    m->device = dev;
     DeviceCtx* ctx = nullptr;
     DQ_CUDA(device_ctx(&ctx));
-    m->sm_count = ctx->sm_count; m->stream = ctx->stream; m->ev0 = ctx->ev0; m->ev1 = ctx->ev1; m->ev2 = ctx->ev2; m->ev3 = ctx->ev3;
-    m->stream2 = ctx->stream2; m->ev_fork = ctx->ev_fork; m->ev_join = ctx->ev_join;
-    m->pin = ctx->pin;
     const CompiledModel& c = m->cm;
     const int nv = c.nv;
     // every table goes into ONE device block with ONE stream-ordered copy (the solve's kernels follow on the same stream)
@@ -254,7 +292,7 @@ static int upload(dq_model* m) {
     const size_t o_s_and = put(c.small_and), o_s_weq = put(c.small_weq), o_s_weq_on = put(c.small_weq_on), o_s_chk = put(c.small_chk),
                  o_s_dom0 = put(dom0_pos);
     DQ_CUDA(m->d_blob.reserve(blob.size()));
-    DQ_CUDA(cudaMemcpyAsync(m->d_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice, m->stream));
+    DQ_CUDA(cudaMemcpyAsync(m->d_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice, ctx->stream));
     uint8_t* base = m->d_blob.p;
     m->t_ent_off = (uint32_t*)(base + o_ent_off); m->t_ent = (uint32_t*)(base + o_ent); m->t_ent_moff = (uint32_t*)(base + o_ent_moff);
     m->t_masks = (uint32_t*)(base + o_masks); m->t_dom0 = (uint32_t*)(base + o_dom0); m->t_order = (uint16_t*)(base + o_order); m->t_pos = (uint16_t*)(base + o_pos);
@@ -262,7 +300,7 @@ static int upload(dq_model* m) {
     m->t_s_and = (uint32_t*)(base + o_s_and); m->t_s_weq = (uint32_t*)(base + o_s_weq); m->t_s_weq_on = (uint32_t*)(base + o_s_weq_on);
     m->t_s_chk = (uint32_t*)(base + o_s_chk); m->t_s_dom0 = (uint32_t*)(base + o_s_dom0);
     DQ_CUDA(m->d_ctrl.reserve(32));
-    m->uploaded = true;
+    m->ctx = ctx;
     return DQ_OK;
 }
 
@@ -294,34 +332,13 @@ template <> struct LevelWords<W64> {
     static DevBuf<W64>& surv(LevelArrays& L) { return L.surv64; }
 };
 
-// Same, for the kernels that are also templated on the domain word type.
-#define DQ_DISPATCH_W(m, W, KERNEL, grid, block, smem, stream, ...)                                       \
-    do {                                                                                                  \
-        if ((m)->cm.has_f) {                                                                              \
-            if ((m)->cm.has_table) KERNEL<true, true, W><<<grid, block, smem, stream>>>(__VA_ARGS__);     \
-            else KERNEL<true, false, W><<<grid, block, smem, stream>>>(__VA_ARGS__);                      \
-        } else {                                                                                          \
-            if ((m)->cm.has_table) KERNEL<false, true, W><<<grid, block, smem, stream>>>(__VA_ARGS__);    \
-            else KERNEL<false, false, W><<<grid, block, smem, stream>>>(__VA_ARGS__);                     \
-        }                                                                                                 \
-    } while (0)
-#define DQ_OCCUPANCY_W(m, W, KERNEL, threads, smem, out)                                               \
-    ((m)->cm.has_f ? ((m)->cm.has_table ? max_ctas_per_sm(KERNEL<true, true, W>, threads, smem, out)  \
-                                        : max_ctas_per_sm(KERNEL<true, false, W>, threads, smem, out)) \
-                   : ((m)->cm.has_table ? max_ctas_per_sm(KERNEL<false, true, W>, threads, smem, out) \
-                                        : max_ctas_per_sm(KERNEL<false, false, W>, threads, smem, out)))
-
-// Picks the template instantiation for the model's feature flags and launches `KERNEL`.
-#define DQ_DISPATCH(m, KERNEL, grid, block, smem, stream, ...)                                            \
-    do {                                                                                                  \
-        if ((m)->cm.has_f) {                                                                              \
-            if ((m)->cm.has_table) KERNEL<true, true><<<grid, block, smem, stream>>>(__VA_ARGS__);        \
-            else KERNEL<true, false><<<grid, block, smem, stream>>>(__VA_ARGS__);                         \
-        } else {                                                                                          \
-            if ((m)->cm.has_table) KERNEL<false, true><<<grid, block, smem, stream>>>(__VA_ARGS__);       \
-            else KERNEL<false, false><<<grid, block, smem, stream>>>(__VA_ARGS__);                        \
-        }                                                                                                 \
-    } while (0)
+// Calls f(has_f, has_table) with the model's feature flags as std::bool_constant, so that f can name the kernel
+// instantiation for them: with_features(m->cm, [&](auto hf, auto ht) { k<hf, ht><<<...>>>(...); }).
+template <class F>
+static auto with_features(const CompiledModel& cm, F&& f) {
+    if (cm.has_f) return cm.has_table ? f(std::true_type{}, std::true_type{}) : f(std::true_type{}, std::false_type{});
+    return cm.has_table ? f(std::false_type{}, std::true_type{}) : f(std::false_type{}, std::false_type{});
+}
 
 template <class K>
 static int max_ctas_per_sm(K kernel, int threads, size_t smem, int* out) {
@@ -332,47 +349,40 @@ static int max_ctas_per_sm(K kernel, int threads, size_t smem, int* out) {
     return DQ_OK;
 }
 
-#define DQ_OCCUPANCY(m, KERNEL, threads, smem, out)                                              \
-    ((m)->cm.has_f ? ((m)->cm.has_table ? max_ctas_per_sm(KERNEL<true, true>, threads, smem, out) \
-                                        : max_ctas_per_sm(KERNEL<true, false>, threads, smem, out)) \
-                   : ((m)->cm.has_table ? max_ctas_per_sm(KERNEL<false, true>, threads, smem, out) \
-                                        : max_ctas_per_sm(KERNEL<false, false>, threads, smem, out)))
-
-
 // FIRST mode on a CLASS_QUEENS model, whole tree in one partition, no node budget: one warp walks the reference's own
 // DFS (k_queens_first_nodes) — the solution, and every value tried on the way counted as the node it is.  One launch, one
 // synchronisation; the generic path's prefix split searches the winning subtree with one warp as well, after paying for
 // the frontier and for the subtrees that hold nothing (20-Queens: 43 ms there).
 static int solve_queens_first(dq_model* m, dq_tree_result* res, int32_t* first_solution) {
     const int N = m->cm.queens_n;
+    DeviceCtx* ctx = m->ctx;
     DQ_CUDA(m->q_first.reserve(32));
     DQ_CUDA(m->d_ctrl.reserve(32));
     unsigned long long* ctrl = m->d_ctrl.p;
-    unsigned long long* h = m->pin;                  // [0] best key [1] nodes, [8..11] the solution bytes
+    auto& P = ctx->pin->queens_first;
+    unsigned long long* h = P.key_nodes;
     h[0] = KEY_NONE; h[1] = 0;
     QueensLaneArgs A;
     A.n = N; A.k = 0; A.part_rank = 0; A.part_count = 1; A.part_level = -1;
     A.records = nullptr; A.record_cap = 0; A.n_records = nullptr; A.cursor = nullptr; A.totals = nullptr; A.dfs_nodes = nullptr;
     A.best_key = ctrl + 3; A.first_out = m->q_first.p;
-    DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
-    DQ_CUDA(cudaMemcpyAsync(ctrl + 3, h, 2 * sizeof(unsigned long long), cudaMemcpyHostToDevice, m->stream));
-    k_queens_first_nodes<<<1, 32, 0, m->stream>>>(A, ctrl + 4);
+    DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+    DQ_CUDA(cudaMemcpyAsync(ctrl + 3, h, sizeof P.key_nodes, cudaMemcpyHostToDevice, ctx->stream));
+    k_queens_first_nodes<<<1, 32, 0, ctx->stream>>>(A, ctrl + 4);
     DQ_CUDA(cudaGetLastError());
-    DQ_CUDA(cudaMemcpyAsync(h, ctrl + 3, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaMemcpyAsync(h + 8, m->q_first.p, 32, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    DQ_CUDA(cudaMemcpyAsync(h, ctrl + 3, sizeof P.key_nodes, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaMemcpyAsync(P.solution, m->q_first.p, sizeof P.solution, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     float ms = 0;
-    DQ_CUDA(cudaEventElapsedTime(&ms, m->ev0, m->ev1));
+    DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     const bool found = h[0] != KEY_NONE;
     res->kernel_ms = ms; res->search_kernel_ms = 0; res->kernel_launches = 1; res->frontier_nodes = 0;
     res->engine_used = DQ_ENGINE_LANE; res->split_depth_used = 0; res->n_prefixes = 1;
     res->n_solutions = found ? 1 : 0; res->n_nodes = h[1]; res->first_key = found ? 0 : KEY_NONE;
     res->outcome = found ? DQ_SAT : DQ_UNSAT;
-    if (found && first_solution) {
-        const uint8_t* sol = reinterpret_cast<const uint8_t*>(h + 8);
-        for (int i = 0; i < N; i++) first_solution[i] = m->cm.values[i][sol[i]];
-    }
+    if (found && first_solution)
+        for (int i = 0; i < N; i++) first_solution[i] = m->cm.values[i][P.solution[i]];
     m->last_queens_first = true; m->last_queens_first_nodes = h[1];
     m->last_n_prefix = 0; m->last_depth = 0;
     return DQ_OK;
@@ -382,6 +392,7 @@ static int solve_queens_first(dq_model* m, dq_tree_result* res, int32_t* first_s
 // kernel queued back to back, one host synchronisation at the end.
 static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_result* res, int32_t* first_solution) {
     const int N = m->cm.queens_n;
+    DeviceCtx* ctx = m->ctx;
     // Split depth: measured per board size on B200 (scripts/sweep_k.py, profiles/r2_queens_split_depth.txt), see below.
     int K = 0;
     // estimated FC-surviving prefixes per depth (sizes the record lists): each level multiplies by about N - 2.2*depth
@@ -433,15 +444,16 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
     }
     const size_t smem = per_warp * bucket_warps;
     if (occ < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
-    const int ctas = occ * m->sm_count;
+    const int ctas = occ * ctx->sm_count;
     DQ_CUDA(m->q_first.reserve(32));
     DQ_CUDA(m->d_ctrl.reserve(32));
     size_t cap = std::max<size_t>(m->q_records.cap, (size_t)std::min(std::max(2.5 * estimate(K), 1024.0), 512.0 * 1024 * 1024));
     // control words live in pinned host memory that outlives the call: the queue below may be replayed as a CUDA graph
-    unsigned long long* h_init = m->pin;              // [32] initial control block
-    uint4* h_root = reinterpret_cast<uint4*>(m->pin + 32);
-    unsigned long long* h_ctrl = m->pin + 40;         // [32] control block read back
-    uint8_t* h_first = reinterpret_cast<uint8_t*>(m->pin + 72);   // [32]
+    auto& P = ctx->pin->queens_lane;
+    unsigned long long* h_init = P.init;
+    uint4* h_root = &P.root;
+    unsigned long long* h_ctrl = P.ctrl;
+    uint8_t* h_first = P.first;
     unsigned long long* ctrl = m->d_ctrl.p;     // [0]=cursor [1]=sols [2]=nodes [3]=best [8+l]=frontier size at depth l
     unsigned long long launches = 0, h_frontier_nodes = 0;
     float ms_total = 0, ms_search = 0;
@@ -473,36 +485,36 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
         // (timing events cannot be read back from inside a graph: the graph is bracketed by ev0 / ev1 from outside, and the
         // per-kernel pair ev2 / ev3 exists only in the call-by-call queue, DQ_TREE_TIME_KERNELS)
         auto enqueue = [&](const bool with_events) -> int {
-            if (with_events) DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
-            DQ_CUDA(cudaMemcpyAsync(ctrl, h_init, 32 * sizeof(unsigned long long), cudaMemcpyHostToDevice, m->stream));
-            DQ_CUDA(cudaMemcpyAsync(buf[0], h_root, sizeof(uint4), cudaMemcpyHostToDevice, m->stream));
+            if (with_events) DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+            DQ_CUDA(cudaMemcpyAsync(ctrl, h_init, sizeof P.init, cudaMemcpyHostToDevice, ctx->stream));
+            DQ_CUDA(cudaMemcpyAsync(buf[0], h_root, sizeof(uint4), cudaMemcpyHostToDevice, ctx->stream));
             // the DFS-first solution needs nothing from the frontier: one warp looks for it on the side stream
-            DQ_CUDA(cudaEventRecord(m->ev_fork, m->stream));
-            DQ_CUDA(cudaStreamWaitEvent(m->stream2, m->ev_fork, 0));
-            k_queens_first_warp<<<1, 32, 0, m->stream2>>>(A);
-            DQ_CUDA(cudaEventRecord(m->ev_join, m->stream2));
+            DQ_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+            DQ_CUDA(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
+            k_queens_first_warp<<<1, 32, 0, ctx->stream2>>>(A);
+            DQ_CUDA(cudaEventRecord(ctx->ev_join, ctx->stream2));
             if (head > 0)
-                k_queens_levels_head<<<1, kQueensBlock, 0, m->stream>>>(A, head, buf[0], buf[1], ctrl + 8, opts->part_rank == 0 ? 1 : 0);
+                k_queens_levels_head<<<1, kQueensBlock, 0, ctx->stream>>>(A, head, buf[0], buf[1], ctrl + 8, opts->part_rank == 0 ? 1 : 0);
             for (int l = head; l < K; l++) {
-                const int grid = (int)std::min<double>(std::max(estimate(l) * N / kQueensBlock, 1.0), (double)m->sm_count * 8);
+                const int grid = (int)std::min<double>(std::max(estimate(l) * N / kQueensBlock, 1.0), (double)ctx->sm_count * 8);
                 const int count_nodes = (l > part_level || opts->part_rank == 0) ? 1 : 0;
                 // wide frontiers: lane per record (k_queens_level_wide); narrow ones: lane per (record, value) pair
                 if (estimate(l) >= 150000.0) {      // (below that the pair kernel's single trip has the shorter latency)
-                    const int wgrid = (int)std::min<double>(std::max(estimate(l) / kQueensBlock, 1.0), (double)m->sm_count * 8);
-                    k_queens_level_wide<<<wgrid, kQueensBlock, 0, m->stream>>>(A, l, buf[l & 1], ctrl + 8 + l, buf[(l + 1) & 1], ctrl + 8 + l + 1,
+                    const int wgrid = (int)std::min<double>(std::max(estimate(l) / kQueensBlock, 1.0), (double)ctx->sm_count * 8);
+                    k_queens_level_wide<<<wgrid, kQueensBlock, 0, ctx->stream>>>(A, l, buf[l & 1], ctrl + 8 + l, buf[(l + 1) & 1], ctrl + 8 + l + 1,
                                                                                 count_nodes, (l == part_level && opts->part_count > 1) ? 1 : 0);
                 } else
-                k_queens_level<<<grid, kQueensBlock, 0, m->stream>>>(A, l, buf[l & 1], ctrl + 8 + l, buf[(l + 1) & 1], ctrl + 8 + l + 1,
+                k_queens_level<<<grid, kQueensBlock, 0, ctx->stream>>>(A, l, buf[l & 1], ctrl + 8 + l, buf[(l + 1) & 1], ctrl + 8 + l + 1,
                                                                        count_nodes, (l == part_level && opts->part_count > 1) ? 1 : 0);
             }
-            if (with_events) DQ_CUDA(cudaEventRecord(m->ev2, m->stream));
-            bucket_kernel<<<ctas, bucket_warps * 32, smem, m->stream>>>(A);
-            if (with_events) DQ_CUDA(cudaEventRecord(m->ev3, m->stream));
-            DQ_CUDA(cudaStreamWaitEvent(m->stream, m->ev_join, 0));
+            if (with_events) DQ_CUDA(cudaEventRecord(ctx->ev2, ctx->stream));
+            bucket_kernel<<<ctas, bucket_warps * 32, smem, ctx->stream>>>(A);
+            if (with_events) DQ_CUDA(cudaEventRecord(ctx->ev3, ctx->stream));
+            DQ_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
             DQ_CUDA(cudaGetLastError());
-            DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, 32 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
-            DQ_CUDA(cudaMemcpyAsync(h_first, m->q_first.p, 32, cudaMemcpyDeviceToHost, m->stream));
-            if (with_events) DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
+            DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof P.ctrl, cudaMemcpyDeviceToHost, ctx->stream));
+            DQ_CUDA(cudaMemcpyAsync(h_first, m->q_first.p, sizeof P.first, cudaMemcpyDeviceToHost, ctx->stream));
+            if (with_events) DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
             return DQ_OK;
         };
         launches += (K - head) + (head > 0 ? 1 : 0) + 2;
@@ -522,9 +534,9 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
             if (seen && (!m->q_exec || memcmp(key, m->q_exec_key, sizeof key) != 0)) {
                 if (m->q_exec) { cudaGraphExecDestroy(m->q_exec); m->q_exec = nullptr; }
                 cudaGraph_t graph = nullptr;
-                if (cudaStreamBeginCapture(m->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+                if (cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
                     const int qrc = enqueue(false);
-                    const cudaError_t ce = cudaStreamEndCapture(m->stream, &graph);
+                    const cudaError_t ce = cudaStreamEndCapture(ctx->stream, &graph);
                     if (qrc == DQ_OK && ce == cudaSuccess && graph && cudaGraphInstantiate(&m->q_exec, graph, 0) == cudaSuccess)
                         memcpy(m->q_exec_key, key, sizeof key);
                     else m->q_exec = nullptr;
@@ -533,8 +545,8 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
                 (void)cudaGetLastError();                      // a failed capture falls back to the plain queue below
             }
             if (m->q_exec && memcmp(key, m->q_exec_key, sizeof key) == 0) {
-                DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
-                if (cudaGraphLaunch(m->q_exec, m->stream) == cudaSuccess) { queued = true; DQ_CUDA(cudaEventRecord(m->ev1, m->stream)); }
+                DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+                if (cudaGraphLaunch(m->q_exec, ctx->stream) == cudaSuccess) { queued = true; DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream)); }
                 else (void)cudaGetLastError();
             }
         }
@@ -542,11 +554,11 @@ static int solve_queens_lane(dq_model* m, const dq_tree_opts* opts, dq_tree_resu
             rc = enqueue(true);
             if (rc != DQ_OK) return rc;
         }
-        DQ_CUDA(cudaStreamSynchronize(m->stream));
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
         float ms = 0;
-        DQ_CUDA(cudaEventElapsedTime(&ms, m->ev0, m->ev1));
+        DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
         ms_total += ms;
-        if (!queued) DQ_CUDA(cudaEventElapsedTime(&ms_search, m->ev2, m->ev3));
+        if (!queued) DQ_CUDA(cudaEventElapsedTime(&ms_search, ctx->ev2, ctx->ev3));
         h_frontier_nodes = h_ctrl[2];
         unsigned long long biggest = 0;
         for (int l = 0; l <= K; l++) biggest = std::max(biggest, h_ctrl[8 + l]);
@@ -608,26 +620,7 @@ int dq_compile(const dq_model_desc* desc, dq_model** out) {
     return DQ_OK;
 }
 
-void dq_free(dq_model* m) {
-    if (!m) return;
-    if (m->multi) { multi_destroy(m->multi); m->multi = nullptr; }
-    if (m->q_exec) { cudaGraphExecDestroy(m->q_exec); m->q_exec = nullptr; }
-    if (m->uploaded) {
-        m->d_blob.release(); m->d_ctrl.release();
-        m->d_sub_nodes.release(); m->d_sol_key.release(); m->d_sol.release(); m->d_lvl_ptrs.release();
-        m->e_out.release(); m->e_prefix.release(); m->e_seq.release();
-        m->q_records.release(); m->q_records2.release(); m->q_first.release();
-        m->b_cells.release(); m->b_solution.release(); m->b_status.release(); m->b_nodes.release();
-        m->s_digest.release(); m->s_ctrl.release(); m->s_hard.release(); m->s_tasks.release(); m->s_snaps.release(); m->s_snap_state.release();
-        m->s_deferred.release();
-        for (auto& l : m->levels) {
-            l.dmask.release(); l.surv.release(); l.dmask64.release(); l.surv64.release(); l.child_off.release(); l.parent_of.release();
-            l.node_off.release(); l.prefixes.release();
-        }
-        m->d_head.release();
-    }
-    delete m;
-}
+void dq_free(dq_model* m) { delete m; }
 
 int dq_model_info(const dq_model* m, int32_t* n_vars, int32_t* max_dom, int32_t* n_arcs, int32_t* model_class) {
     if (!m) { g_err = "null model"; return DQ_ERR_INVALID; }
@@ -669,6 +662,7 @@ template <typename W>
 static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_result* res, int32_t* first_solution, EnumRequest* er,
                               const bool count_all) {
     const int nv = m->cm.nv;
+    DeviceCtx* ctx = m->ctx;
     int rc = DQ_OK;
     TreeModelDevT<W> M = dev_model_t<W>(m);
     m->last_wide = sizeof(W) == 8;
@@ -678,13 +672,13 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
     if (wpc < 1) { g_err = "model state exceeds shared memory"; return DQ_ERR_UNSUPPORTED; }
     const size_t smem = wbytes * wpc;
     int occ = 0;
-    rc = DQ_OCCUPANCY_W(m, W, k_tree_dfs, wpc * 32, smem, &occ);
+    rc = with_features(m->cm, [&](auto hf, auto ht) { return max_ctas_per_sm(k_tree_dfs<hf, ht, W>, wpc * 32, smem, &occ); });
     if (rc != DQ_OK) return rc;
     int occ_e = 0;
-    rc = DQ_OCCUPANCY_W(m, W, k_expand, wpc * 32, smem, &occ_e);
+    rc = with_features(m->cm, [&](auto hf, auto ht) { return max_ctas_per_sm(k_expand<hf, ht, W>, wpc * 32, smem, &occ_e); });
     if (rc != DQ_OK) return rc;
     if (occ < 1 || occ_e < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
-    const long long resident_warps = (long long)occ * m->sm_count * wpc;
+    const long long resident_warps = (long long)occ * ctx->sm_count * wpc;
     const int max_depth = nv - 1;
     const int want_depth = opts->split_depth > 0 ? std::min(opts->split_depth, max_depth) : -1;
     // lane-per-subtree counting (dq_lane_tree.cuh) for small models whose pair filters are plain AND masks
@@ -699,7 +693,7 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
     }
     // enough prefixes for 24 rounds of the resident warps — or, one subtree per lane, one round of the resident lanes
     // (2 or 4 rounds are no faster: profiles/r2_generic_lane_tree.txt)
-    const long long want_prefixes = (lanes ? (long long)occ_l * m->sm_count * kLaneTreeThreads : resident_warps * 24) * opts->part_count;
+    const long long want_prefixes = (lanes ? (long long)occ_l * ctx->sm_count * kLaneTreeThreads : resident_warps * 24) * opts->part_count;
 
     if (er) {
         DQ_CUDA(m->e_out.reserve(std::max<size_t>((size_t)er->cap * nv, 1)));
@@ -708,8 +702,8 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
     }
     unsigned long long* ctrl = m->d_ctrl.p;   // [0]=cursor [1]=sols [2]=nodes [3]=best [4]=scan children [5]=scan nodes [6]=probe gave up [7]=enumerated
     unsigned long long h_ctrl[8] = {0, 0, 0, KEY_NONE, 0, 0, 0, 0};
-    DQ_CUDA(cudaMemcpyAsync(ctrl, h_ctrl, sizeof h_ctrl, cudaMemcpyHostToDevice, m->stream));
-    DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
+    DQ_CUDA(cudaMemcpyAsync(ctrl, h_ctrl, sizeof h_ctrl, cudaMemcpyHostToDevice, ctx->stream));
+    DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
 
     if ((int)m->levels.size() < nv + 1) m->levels.resize(nv + 1);   // sized up front: references below stay valid
     m->levels[0].n = 1;
@@ -736,13 +730,13 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
         const bool by_lane = lanes && !node_budget && mine >= 2048;          // (a handful of prefixes: the warp-cooperative engines)
         const long long per_sm = by_lane ? occ_l : (small ? socc : occ);
         const int w_cta = by_lane ? kLaneTreeThreads : (small ? kWarpsPerCta : wpc);     // result slots per CTA: lanes or warps
-        const long long ctas = std::max<long long>(1, std::min<long long>((long long)((mine + w_cta - 1) / w_cta), per_sm * m->sm_count));
+        const long long ctas = std::max<long long>(1, std::min<long long>((long long)((mine + w_cta - 1) / w_cta), per_sm * ctx->sm_count));
         n_warps = ctas * w_cta;
         DQ_CUDA(m->d_sub_nodes.reserve(n_prefix));
         DQ_CUDA(m->d_sol_key.reserve(n_warps));
         DQ_CUDA(m->d_sol.reserve((size_t)n_warps * nv));
-        DQ_CUDA(cudaMemsetAsync(m->d_sub_nodes.p, 0, n_prefix * sizeof(unsigned long long), m->stream));
-        DQ_CUDA(cudaMemsetAsync(m->d_sol_key.p, 0xFF, n_warps * sizeof(unsigned long long), m->stream));
+        DQ_CUDA(cudaMemsetAsync(m->d_sub_nodes.p, 0, n_prefix * sizeof(unsigned long long), ctx->stream));
+        DQ_CUDA(cudaMemsetAsync(m->d_sol_key.p, 0xFF, n_warps * sizeof(unsigned long long), ctx->stream));
         TreeDfsArgs A;
         A.prefixes = m->levels[at_depth].prefixes.p; A.depth = at_depth; A.n_prefix = n_prefix;
         A.part_rank = part_rank; A.part_count = part_count; A.count_all = count_all ? 1 : 0;
@@ -755,16 +749,16 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
             SmallTablesDev ST;
             ST.nv = nv; ST.kmax = m->cm.kmax; ST.t_and = m->t_s_and; ST.t_weq = m->t_s_weq; ST.t_weq_on = m->t_s_weq_on;
             ST.t_chk = m->t_s_chk; ST.dom0_pos = m->t_s_dom0; ST.order = m->t_order;
-            k_tree_lanes<<<(int)ctas, kLaneTreeThreads, lane_tree_smem(nv, m->cm.kmax), m->stream>>>(ST, A);
+            k_tree_lanes<<<(int)ctas, kLaneTreeThreads, lane_tree_smem(nv, m->cm.kmax), ctx->stream>>>(ST, A);
             res->engine_used = DQ_ENGINE_LANE;
         } else if (small) {
             SmallTablesDev ST;
             ST.nv = nv; ST.kmax = m->cm.kmax; ST.t_and = m->t_s_and; ST.t_weq = m->t_s_weq; ST.t_weq_on = m->t_s_weq_on;
             ST.t_chk = m->t_s_chk; ST.dom0_pos = m->t_s_dom0; ST.order = m->t_order;
-            if (m->cm.has_f) k_tree_small<true><<<(int)ctas, kWarpsPerCta * 32, ssm, m->stream>>>(ST, A);
-            else k_tree_small<false><<<(int)ctas, kWarpsPerCta * 32, ssm, m->stream>>>(ST, A);
+            if (m->cm.has_f) k_tree_small<true><<<(int)ctas, kWarpsPerCta * 32, ssm, ctx->stream>>>(ST, A);
+            else k_tree_small<false><<<(int)ctas, kWarpsPerCta * 32, ssm, ctx->stream>>>(ST, A);
             res->engine_used = DQ_ENGINE_REG;
-        } else DQ_DISPATCH_W(m, W, k_tree_dfs, (int)ctas, wpc * 32, smem, m->stream, M, A);
+        } else with_features(m->cm, [&](auto hf, auto ht) { k_tree_dfs<hf, ht, W><<<(int)ctas, wpc * 32, smem, ctx->stream>>>(M, A); });
         launches++;
         DQ_CUDA(cudaGetLastError());
         return DQ_OK;
@@ -778,14 +772,14 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
     if (want_depth < 0 && opts->part_count == 1 && !er) {
         rc = launch_dfs(0, 1, 0, 1, kProbeNodes);
         if (rc != DQ_OK) return rc;
-        DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
-        DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof h_ctrl, cudaMemcpyDeviceToHost, m->stream));
-        DQ_CUDA(cudaStreamSynchronize(m->stream));
+        DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+        DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof h_ctrl, cudaMemcpyDeviceToHost, ctx->stream));
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
         if (h_ctrl[6] == 0) probed = true;
         else {
             const unsigned long long z[8] = {0, 0, 0, KEY_NONE, 0, 0, 0, 0};
             memcpy(h_ctrl, z, sizeof z);
-            DQ_CUDA(cudaMemcpyAsync(ctrl, h_ctrl, sizeof h_ctrl, cudaMemcpyHostToDevice, m->stream));
+            DQ_CUDA(cudaMemcpyAsync(ctrl, h_ctrl, sizeof h_ctrl, cudaMemcpyHostToDevice, ctx->stream));
         }
     }
 
@@ -803,17 +797,8 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
         const size_t off_base = (bytes + 15) & ~(size_t)15;
         bytes = off_base + 2 * (size_t)nv * sizeof(W);
         if (m->d_head.cap < bytes || m->head_levels < head_max + 1) {
-            for (auto& L : m->levels) {                       // views of the old slab go first
-                if (L.dmask.view) L.dmask.release();
-                if (L.surv.view) L.surv.release();
-                if (L.dmask64.view) L.dmask64.release();
-                if (L.surv64.view) L.surv64.release();
-                if (L.child_off.view) L.child_off.release();
-                if (L.parent_of.view) L.parent_of.release();
-                if (L.node_off.view) L.node_off.release();
-                if (L.prefixes.view) L.prefixes.release();
-            }
-            DQ_CUDA(cudaStreamSynchronize(m->stream));
+            for (auto& L : m->levels) L.release_views();     // views of the old slab go first
+            DQ_CUDA(cudaStreamSynchronize(ctx->stream));
             DQ_CUDA(m->d_head.reserve(bytes));
             m->head_levels = head_max + 1;
         }
@@ -837,21 +822,24 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
             if (L.prefixes.cap < (size_t)kHeadCap * std::max(l, 1) || L.prefixes.view) L.prefixes.set_view(H.prefixes, (size_t)kHeadCap * std::max(l, 1)); else H.prefixes = L.prefixes.p;
         }
         HeadLevel<W>* d_tab = reinterpret_cast<HeadLevel<W>*>(m->d_head.p + off_tab);
-        DQ_CUDA(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(HeadLevel<W>), cudaMemcpyHostToDevice, m->stream));
+        DQ_CUDA(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(HeadLevel<W>), cudaMemcpyHostToDevice, ctx->stream));
         DQ_CUDA(m->d_lvl_ptrs.reserve((size_t)(kHeadMaxLevels + 8) * 8 + 4096));
         unsigned long long* d_out = reinterpret_cast<unsigned long long*>(m->d_lvl_ptrs.p);
         int occ_h = 0;
-        rc = DQ_OCCUPANCY_W(m, W, k_expand_head, 32, wbytes, &occ_h);      // (also lifts the 48 KB dynamic shared-memory limit)
+        // (also lifts the 48 KB dynamic shared-memory limit)
+        rc = with_features(m->cm, [&](auto hf, auto ht) { return max_ctas_per_sm(k_expand_head<hf, ht, W>, 32, wbytes, &occ_h); });
         if (rc != DQ_OK) return rc;
         W* base_D = reinterpret_cast<W*>(m->d_head.p + off_base);
-        DQ_DISPATCH_W(m, W, k_expand_head, 1, 32, wbytes, m->stream, M, d_tab, head_max, base_D, base_D + nv, d_out);
+        with_features(m->cm, [&](auto hf, auto ht) {
+            k_expand_head<hf, ht, W><<<1, 32, wbytes, ctx->stream>>>(M, d_tab, head_max, base_D, base_D + nv, d_out);
+        });
         launches++;
-        unsigned long long* h_out = m->pin + 80;             // (pinned; 40 words are free there: [80, 119))
-        const int n_read = std::min(4 + head_max + 1, 38);
-        DQ_CUDA(cudaMemcpyAsync(h_out, d_out, (size_t)n_read * 8, cudaMemcpyDeviceToHost, m->stream));
+        unsigned long long* h_out = ctx->pin->head;
+        const int n_read = std::min(4 + head_max + 1, (int)std::size(ctx->pin->head));
+        DQ_CUDA(cudaMemcpyAsync(h_out, d_out, (size_t)n_read * 8, cudaMemcpyDeviceToHost, ctx->stream));
         std::vector<unsigned long long> h_all;
-        if (4 + head_max + 1 > n_read) { h_all.resize(4 + head_max + 1); DQ_CUDA(cudaMemcpyAsync(h_all.data(), d_out, h_all.size() * 8, cudaMemcpyDeviceToHost, m->stream)); }
-        DQ_CUDA(cudaStreamSynchronize(m->stream));
+        if (4 + head_max + 1 > n_read) { h_all.resize(4 + head_max + 1); DQ_CUDA(cudaMemcpyAsync(h_all.data(), d_out, h_all.size() * 8, cudaMemcpyDeviceToHost, ctx->stream)); }
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
         DQ_CUDA(cudaGetLastError());
         const unsigned long long* ho = h_all.empty() ? h_out : h_all.data();
         depth = (int)ho[0];
@@ -870,12 +858,14 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
         DevBuf<W>& Lsurv = LevelWords<W>::surv(L);
         DQ_CUDA(Ldmask.reserve(n)); DQ_CUDA(Lsurv.reserve(n)); DQ_CUDA(L.child_off.reserve(n)); DQ_CUDA(L.node_off.reserve(n));
         const int grid = (n + wpc - 1) / wpc;
-        DQ_DISPATCH_W(m, W, k_expand, grid, wpc * 32, smem, m->stream, M, L.prefixes.p, depth, n, Ldmask.p, Lsurv.p);
-        k_scan_level<W><<<1, 1024, 0, m->stream>>>(Ldmask.p, Lsurv.p, n, L.child_off.p, L.node_off.p, ctrl + 4);
+        with_features(m->cm, [&](auto hf, auto ht) {
+            k_expand<hf, ht, W><<<grid, wpc * 32, smem, ctx->stream>>>(M, L.prefixes.p, depth, n, Ldmask.p, Lsurv.p);
+        });
+        k_scan_level<W><<<1, 1024, 0, ctx->stream>>>(Ldmask.p, Lsurv.p, n, L.child_off.p, L.node_off.p, ctrl + 4);
         launches += 2;
-        unsigned long long* tot = m->pin + 76;              // (pinned: a pageable target costs a staging copy per level)
-        DQ_CUDA(cudaMemcpyAsync(tot, ctrl + 4, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
-        DQ_CUDA(cudaStreamSynchronize(m->stream));
+        unsigned long long* tot = ctx->pin->level_totals;
+        DQ_CUDA(cudaMemcpyAsync(tot, ctrl + 4, sizeof ctx->pin->level_totals, cudaMemcpyDeviceToHost, ctx->stream));
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
         shallow_nodes += tot[1];
         if (tot[0] == 0) { empty = true; depth++; m->levels[depth].n = 0; break; }
         if (tot[0] > 0x7FFFFFFFull / (unsigned)(depth + 1)) { g_err = "frontier too large"; return DQ_ERR_NOMEM; }
@@ -883,7 +873,7 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
         C.n = (int)tot[0];
         DQ_CUDA(C.prefixes.reserve((size_t)C.n * (depth + 1)));
         DQ_CUDA(C.parent_of.reserve(C.n));
-        k_write_children<W><<<(n + 255) / 256, 256, 0, m->stream>>>(L.prefixes.p, depth, n, Lsurv.p, L.child_off.p, C.prefixes.p, C.parent_of.p);
+        k_write_children<W><<<(n + 255) / 256, 256, 0, ctx->stream>>>(L.prefixes.p, depth, n, Lsurv.p, L.child_off.p, C.prefixes.p, C.parent_of.p);
         launches++;
         depth++;
     }
@@ -898,22 +888,22 @@ static int solve_tree_generic(dq_model* m, const dq_tree_opts* opts, dq_tree_res
 
     // ---- subtree DFS ----
     if (n_prefix && !probed) {
-        DQ_CUDA(cudaEventRecord(m->ev2, m->stream));
+        DQ_CUDA(cudaEventRecord(ctx->ev2, ctx->stream));
         rc = launch_dfs(depth, n_prefix, opts->part_rank, opts->part_count, 0ull);
         if (rc != DQ_OK) return rc;
-        DQ_CUDA(cudaEventRecord(m->ev3, m->stream));
+        DQ_CUDA(cudaEventRecord(ctx->ev3, ctx->stream));
     }
     if (!probed) {
-        DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
-        DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof h_ctrl, cudaMemcpyDeviceToHost, m->stream));
-        DQ_CUDA(cudaStreamSynchronize(m->stream));
+        DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+        DQ_CUDA(cudaMemcpyAsync(h_ctrl, ctrl, sizeof h_ctrl, cudaMemcpyDeviceToHost, ctx->stream));
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     float ms = 0;
-    DQ_CUDA(cudaEventElapsedTime(&ms, m->ev0, m->ev1));
+    DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     res->kernel_ms = ms;
     res->kernel_launches = launches;
     if (n_prefix && !probed) {                            // the subtree search alone (the frontier levels are the rest)
-        DQ_CUDA(cudaEventElapsedTime(&ms, m->ev2, m->ev3));
+        DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev2, ctx->ev3));
         res->search_kernel_ms = ms;
     }
 
@@ -1027,7 +1017,8 @@ int dq_enumerate_solutions(dq_model* m, const dq_tree_opts* opts, dq_tree_result
 int dq_tree_nodes_upto(dq_model* m, uint64_t key, uint64_t* nodes) {
     if (!m || !nodes) { g_err = "null argument"; return DQ_ERR_INVALID; }
     *nodes = 0;
-    if (!m->uploaded) { g_err = "no solve to account for"; return DQ_ERR_INVALID; }
+    if (!m->ctx) { g_err = "no solve to account for"; return DQ_ERR_INVALID; }
+    DeviceCtx* ctx = m->ctx;
     if (m->last_queens_first) { *nodes = m->last_queens_first_nodes; return DQ_OK; }     // (one partition: the whole count is its share)
     const int depth = m->last_depth;
     const unsigned long long n_prefix = m->last_n_prefix;
@@ -1068,13 +1059,13 @@ int dq_tree_nodes_upto(dq_model* m, uint64_t key, uint64_t* nodes) {
                 lp[l].dmask = wide ? (const void*)L.dmask64.p : (const void*)L.dmask.p;
             }
             DQ_CUDA(m->d_lvl_ptrs.reserve((size_t)(depth + 1) * sizeof(LevelPtrs) + 8));
-            DQ_CUDA(cudaMemcpyAsync(m->d_lvl_ptrs.p + 8, lp.data(), lp.size() * sizeof(LevelPtrs), cudaMemcpyHostToDevice, m->stream));
-            k_nodes_upto<<<1, 32, 0, m->stream>>>(reinterpret_cast<const LevelPtrs*>(m->d_lvl_ptrs.p + 8), depth, key,
+            DQ_CUDA(cudaMemcpyAsync(m->d_lvl_ptrs.p + 8, lp.data(), lp.size() * sizeof(LevelPtrs), cudaMemcpyHostToDevice, ctx->stream));
+            k_nodes_upto<<<1, 32, 0, ctx->stream>>>(reinterpret_cast<const LevelPtrs*>(m->d_lvl_ptrs.p + 8), depth, key,
                                                   m->levels[depth].prefixes.p + key * (size_t)depth, wide ? 1 : 0,
                                                   reinterpret_cast<unsigned long long*>(m->d_lvl_ptrs.p));
             unsigned long long above = 0;
-            DQ_CUDA(cudaMemcpyAsync(&above, m->d_lvl_ptrs.p, sizeof above, cudaMemcpyDeviceToHost, m->stream));
-            DQ_CUDA(cudaStreamSynchronize(m->stream));
+            DQ_CUDA(cudaMemcpyAsync(&above, m->d_lvl_ptrs.p, sizeof above, cudaMemcpyDeviceToHost, ctx->stream));
+            DQ_CUDA(cudaStreamSynchronize(ctx->stream));
             total += above;
         }
     }
@@ -1213,33 +1204,34 @@ static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int
         g_err = "the lane batch engine serves the 9x9 Sudoku class only"; return DQ_ERR_UNSUPPORTED;
     }
     const int nv = m->cm.nv;
+    DeviceCtx* ctx = m->ctx;
     const TreeModelDev M = dev_model(m);
     const size_t smem = warp_state_bytes(nv, M.trail) * kWarpsPerCta;
     if (smem > 200 * 1024) { g_err = "model state exceeds shared memory"; return DQ_ERR_UNSUPPORTED; }
     int occ = 0;
-    int rc = DQ_OCCUPANCY(m, k_batch_cells, kWarpsPerCta * 32, smem, &occ);
+    int rc = with_features(m->cm, [&](auto hf, auto ht) { return max_ctas_per_sm(k_batch_cells<hf, ht>, kWarpsPerCta * 32, smem, &occ); });
     if (rc != DQ_OK) return rc;
     if (occ < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
     unsigned long long* ctrl = m->d_ctrl.p;
-    DQ_CUDA(cudaMemsetAsync(ctrl, 0, 8 * sizeof(unsigned long long), m->stream));
+    DQ_CUDA(cudaMemsetAsync(ctrl, 0, 8 * sizeof(unsigned long long), ctx->stream));
     BatchCellsArgs A;
     A.idx_list = idx_list;
     A.cells = cells_dev; A.n = n; A.stride = stride; A.cell_lut = m->t_cell_lut; A.values = m->t_values;
     A.sizes = m->t_sizes; A.n_sizes = m->n_sizes; A.budget = opts ? opts->node_budget : 0;
     A.cursor = ctrl; A.solution = sol_dev; A.nodes = nodes_dev; A.status = status_dev; A.totals = ctrl + 1;
-    long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)occ * m->sm_count);
+    long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)occ * ctx->sm_count);
     if (ctas < 1) ctas = 1;
-    if (timed) DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
-    DQ_DISPATCH(m, k_batch_cells, (int)ctas, kWarpsPerCta * 32, smem, m->stream, M, A);
+    if (timed) DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+    with_features(m->cm, [&](auto hf, auto ht) { k_batch_cells<hf, ht><<<(int)ctas, kWarpsPerCta * 32, smem, ctx->stream>>>(M, A); });
     DQ_CUDA(cudaGetLastError());
     if (!timed) return DQ_OK;
-    DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
+    DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
     unsigned long long h[8];
-    DQ_CUDA(cudaMemcpyAsync(h, ctrl, sizeof h, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    DQ_CUDA(cudaMemcpyAsync(h, ctrl, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     if (st) {
         float ms = 0;
-        DQ_CUDA(cudaEventElapsedTime(&ms, m->ev0, m->ev1));
+        DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
         st->n_sat = h[1]; st->n_unsat = h[2]; st->n_budget = h[3]; st->total_nodes = h[4];
         st->kernel_ms = ms; st->kernel_launches = 1;
     }
@@ -1252,6 +1244,7 @@ static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int
 // engine afterwards.
 static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, int32_t stride, const dq_batch_opts* opts,
                             uint8_t* sol_dev, unsigned long long* nodes_dev, uint8_t* status_dev, dq_batch_stats* st) {
+    DeviceCtx* ctx = m->ctx;
     int rc = DQ_OK;
     // the number of pieces handed over at the tail does not shrink with the batch: generous floors (64 MB + 192 MB)
     const unsigned long long task_cap = std::max<unsigned long long>(1u << 24, std::min<unsigned long long>(8ull * n, 1ull << 26));   // (16 B each; a task per 512 counted nodes and more)
@@ -1261,11 +1254,11 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     DQ_CUDA(m->s_digest.reserve(n)); DQ_CUDA(m->s_hard.reserve(2 * (size_t)n)); DQ_CUDA(m->s_ctrl.reserve(16));
     DQ_CUDA(m->s_tasks.reserve(task_cap)); DQ_CUDA(m->s_snaps.reserve(snap_cap * kSnapWords)); DQ_CUDA(m->s_snap_state.reserve(snap_cap));
     unsigned long long* ctrl = m->s_ctrl.p;       // SkCtrl words
-    DQ_CUDA(cudaMemsetAsync(ctrl, 0, 16 * sizeof(unsigned long long), m->stream));
-    DQ_CUDA(cudaMemsetAsync(m->s_snap_state.p, 0, snap_cap * sizeof(uint32_t), m->stream));
+    DQ_CUDA(cudaMemsetAsync(ctrl, 0, 16 * sizeof(unsigned long long), ctx->stream));
+    DQ_CUDA(cudaMemsetAsync(m->s_snap_state.p, 0, snap_cap * sizeof(uint32_t), ctx->stream));
     // task records double as "published" flags: the part the previous call used must read zero again
     const unsigned long long dirty = fresh_pool ? m->s_tasks.cap : std::min<unsigned long long>(m->s_tasks_used, m->s_tasks.cap);
-    if (dirty) DQ_CUDA(cudaMemsetAsync(m->s_tasks.p, 0, dirty * sizeof(SudokuTask), m->stream));
+    if (dirty) DQ_CUDA(cudaMemsetAsync(m->s_tasks.p, 0, dirty * sizeof(SudokuTask), ctx->stream));
     SudokuArgs A;
     A.digest = m->s_digest.p; A.n = n; A.stride = stride; A.cells = cells_dev; A.solution = sol_dev; A.nodes = nodes_dev;
     A.status = status_dev; A.hard = m->s_hard.p; A.tasks = m->s_tasks.p; A.task_cap = task_cap;
@@ -1273,22 +1266,22 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     A.force_donate = opts && opts->task_nodes > 0 ? (unsigned)opts->task_nodes : 0u;
     A.first_budget = n >= 400000 ? 3072u : 1024u;   // measured at 1 M: 1024 -> 32.7 ms, 2048 -> 30.3, 3072 -> 29.5; 125 k shards: flat 512-1024 (7.2 ms), 1536 -> 7.6
     if (A.force_donate) A.first_budget = std::min(A.first_budget, 4u * A.force_donate);       // tests: push work through the task path
-    const long long sms = m->sm_count;
-    DQ_CUDA(cudaEventRecord(m->ev0, m->stream));
+    const long long sms = ctx->sm_count;
+    DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
     {
         int occ_d = 0;
         rc = max_ctas_per_sm(k_sudoku_digest, kDigestTile, kDigestSmem, &occ_d);
         if (rc != DQ_OK) return rc;
         const long long tiles = (n + kDigestTile - 1) / kDigestTile;
-        k_sudoku_digest<<<(unsigned)std::max<long long>(1, std::min<long long>(tiles, (long long)std::max(occ_d, 1) * sms)), kDigestTile, kDigestSmem, m->stream>>>(
+        k_sudoku_digest<<<(unsigned)std::max<long long>(1, std::min<long long>(tiles, (long long)std::max(occ_d, 1) * sms)), kDigestTile, kDigestSmem, ctx->stream>>>(
             cells_dev, n, stride, m->s_digest.p, ctrl + SKC_MAX_BLANK);
     }
     // The lanes' stacks are sized for the instance with the most blanks (one 8-byte read-back after the digest, ~20 us):
     // with 30 givens that is 51 levels instead of 81, 354 bytes of shared memory per lane instead of 414, and a fifth CTA
     // (20 warps instead of 16) on every SM.
-    unsigned long long* h_blank = m->pin + 117;
-    DQ_CUDA(cudaMemcpyAsync(h_blank, ctrl + SKC_MAX_BLANK, sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    unsigned long long* h_blank = &ctx->pin->sudoku_max_blank;
+    DQ_CUDA(cudaMemcpyAsync(h_blank, ctrl + SKC_MAX_BLANK, sizeof *h_blank, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     const int levels = (int)std::min<unsigned long long>(std::max<unsigned long long>(*h_blank, 1), 81);
     const size_t smem = offsetof(SudokuSmem, stk) + (size_t)levels * kSudokuBlock * sizeof(uint16_t);
     const size_t smem_strong = sudoku_strong_smem(levels);       // (30 givens: 36 KB per CTA, 24 warps per SM instead of 16)
@@ -1301,28 +1294,28 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     if (rc != DQ_OK) return rc;
     if (occ_first < 1 || occ_count < 1 || occ_walk < 1 || occ_strong < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
     const long long ctas_first = std::max<long long>(1, std::min<long long>(occ_first * sms, (long long)((n + kSudokuBlock - 1) / kSudokuBlock)));
-    k_sudoku_first<<<(unsigned)ctas_first, kSudokuBlock, smem, m->stream>>>(A);
+    k_sudoku_first<<<(unsigned)ctas_first, kSudokuBlock, smem, ctx->stream>>>(A);
     // the hard list's length stays on the device: the next three kernels are sized for the machine and find it in ctrl
-    k_sudoku_strong<<<(unsigned)(occ_strong * sms), 128, smem_strong, m->stream>>>(A);
+    k_sudoku_strong<<<(unsigned)(occ_strong * sms), 128, smem_strong, ctx->stream>>>(A);
     // Host-buffer call without a node budget: every solution is final here (what follows only counts nodes), so the
     // 81 bytes per instance go home on the side stream while the counting stage runs.
     if (m->early_sol_host && !A.user_budget) {
-        DQ_CUDA(cudaEventRecord(m->ev_fork, m->stream));
-        DQ_CUDA(cudaStreamWaitEvent(m->stream2, m->ev_fork, 0));
-        DQ_CUDA(cudaMemcpyAsync(m->early_sol_host, sol_dev, (size_t)n * stride, cudaMemcpyDeviceToHost, m->stream2));
-        DQ_CUDA(cudaEventRecord(m->ev_join, m->stream2));
+        DQ_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+        DQ_CUDA(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
+        DQ_CUDA(cudaMemcpyAsync(m->early_sol_host, sol_dev, (size_t)n * stride, cudaMemcpyDeviceToHost, ctx->stream2));
+        DQ_CUDA(cudaEventRecord(ctx->ev_join, ctx->stream2));
         m->early_sol_done = true;
     }
-    k_sudoku_walk<<<(unsigned)std::min<long long>(occ_walk * sms, (long long)((n + kSudokuBlock - 1) / kSudokuBlock)), kSudokuBlock, smem, m->stream>>>(A);
-    k_sudoku_count<<<(unsigned)(occ_count * sms), kSudokuBlock, smem, m->stream>>>(A);
-    k_sudoku_finish<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(A, ctrl + SKC_TOTALS);
+    k_sudoku_walk<<<(unsigned)std::min<long long>(occ_walk * sms, (long long)((n + kSudokuBlock - 1) / kSudokuBlock)), kSudokuBlock, smem, ctx->stream>>>(A);
+    k_sudoku_count<<<(unsigned)(occ_count * sms), kSudokuBlock, smem, ctx->stream>>>(A);
+    k_sudoku_finish<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(A, ctrl + SKC_TOTALS);
     DQ_CUDA(m->s_deferred.reserve(n));
-    k_sudoku_collect_deferred<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(status_dev, n, m->s_deferred.p, ctrl + 10);
+    k_sudoku_collect_deferred<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(status_dev, n, m->s_deferred.p, ctrl + 10);
     unsigned long long launches = 7;
     DQ_CUDA(cudaGetLastError());
     unsigned long long hc[16];
-    DQ_CUDA(cudaMemcpyAsync(hc, ctrl, sizeof hc, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    DQ_CUDA(cudaMemcpyAsync(hc, ctrl, sizeof hc, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     m->s_tasks_used = std::min(hc[SKC_RESERVE], task_cap);
     if (hc[SKC_ERROR] & 2) { g_err = "sudoku task pool overflow"; return DQ_ERR_NOMEM; }
     if (hc[SKC_ERROR] || hc[SKC_OUTSTANDING]) {
@@ -1331,7 +1324,7 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
     }
     const unsigned long long n_def = hc[10];
     unsigned long long hw[8] = {0};
-    if (m->early_sol_done) DQ_CUDA(cudaStreamWaitEvent(m->stream, m->ev_join, 0));
+    if (m->early_sol_done) DQ_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
     if (n_def) {
         m->early_sol_done = false;                 // (the generic engine is about to write the deferred instances' solutions)
         dq_batch_opts o2 = opts ? *opts : dq_batch_opts{0, 0, 0};
@@ -1340,12 +1333,12 @@ static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, in
         if (rc != DQ_OK) return rc;
         launches++;
     }
-    DQ_CUDA(cudaEventRecord(m->ev1, m->stream));
-    if (n_def) DQ_CUDA(cudaMemcpyAsync(hw, m->d_ctrl.p, sizeof hw, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+    if (n_def) DQ_CUDA(cudaMemcpyAsync(hw, m->d_ctrl.p, sizeof hw, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     if (st) {
         float ms = 0;
-        DQ_CUDA(cudaEventElapsedTime(&ms, m->ev0, m->ev1));
+        DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
         const unsigned long long* ht = hc + SKC_TOTALS;
         st->n_sat = ht[0] + hw[1]; st->n_unsat = ht[1] + hw[2]; st->n_budget = ht[2] + hw[3]; st->total_nodes = ht[3] + hw[4];
         st->kernel_ms = ms; st->kernel_launches = launches;
@@ -1371,10 +1364,11 @@ int dq_solve_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t s
     if (!cells || !solution || !nodes || !status) { g_err = "null buffer"; return DQ_ERR_INVALID; }
     int rc = upload(m);
     if (rc != DQ_OK) return rc;
+    DeviceCtx* ctx = m->ctx;
     const size_t bytes = (size_t)n * stride;
     DQ_CUDA(m->b_cells.reserve(bytes)); DQ_CUDA(m->b_solution.reserve(bytes));
     DQ_CUDA(m->b_status.reserve(n)); DQ_CUDA(m->b_nodes.reserve(n));
-    DQ_CUDA(cudaMemcpyAsync(m->b_cells.p, cells, bytes, cudaMemcpyHostToDevice, m->stream));
+    DQ_CUDA(cudaMemcpyAsync(m->b_cells.p, cells, bytes, cudaMemcpyHostToDevice, ctx->stream));
     // (only into page-locked memory: an "asynchronous" copy into pageable memory holds the calling thread until it is
     // done, which would park the pipeline between its stages)
     cudaPointerAttributes pa;
@@ -1383,11 +1377,11 @@ int dq_solve_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t s
     m->early_sol_host = pinned ? solution : nullptr; m->early_sol_done = false;
     rc = run_batch_cells(m, m->b_cells.p, n, stride, opts, m->b_solution.p, m->b_nodes.p, m->b_status.p, stats);
     m->early_sol_host = nullptr;
-    if (rc != DQ_OK) { cudaStreamSynchronize(m->stream2); return rc; }     // (nothing may still be writing the caller's buffer)
-    if (!m->early_sol_done) DQ_CUDA(cudaMemcpyAsync(solution, m->b_solution.p, bytes, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaMemcpyAsync(nodes, m->b_nodes.p, (size_t)n * 8, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaMemcpyAsync(status, m->b_status.p, (size_t)n, cudaMemcpyDeviceToHost, m->stream));
-    DQ_CUDA(cudaStreamSynchronize(m->stream));
+    if (rc != DQ_OK) { cudaStreamSynchronize(ctx->stream2); return rc; }     // (nothing may still be writing the caller's buffer)
+    if (!m->early_sol_done) DQ_CUDA(cudaMemcpyAsync(solution, m->b_solution.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaMemcpyAsync(nodes, m->b_nodes.p, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaMemcpyAsync(status, m->b_status.p, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CUDA(cudaStreamSynchronize(ctx->stream));
     if (stats) { stats->h2d_bytes = bytes; stats->d2h_bytes = bytes + (size_t)n * 9; }
     return DQ_OK;
 }
@@ -1432,8 +1426,8 @@ static int run_graphs_lane(int nv, int k, const int64_t* edge_off, const GraphBa
     // pass 1 over the edge lists: how long an overflow list do rows of 8 slots leave behind?  (one 8-byte read-back)
     long long actas = std::max<long long>(1, std::min<long long>((n + kAdjWarpsPerCta - 1) / kAdjWarpsPerCta, (long long)occ_a * sms));
     k_graphs_adjacency<true><<<(unsigned)actas, kAdjWarpsPerCta * 32, graphs_adj_warp_bytes(A.nvp, A.stride, stage_cap) * kAdjWarpsPerCta, s>>>(A, stage_cap);
-    unsigned long long* h_over = ctx->pin + 128 - 9;
-    DQ_CUDA(cudaMemcpyAsync(h_over, d_ctrl + 6, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    unsigned long long* h_over = &ctx->pin->graphs_over;
+    DQ_CUDA(cudaMemcpyAsync(h_over, d_ctrl + 6, sizeof *h_over, cudaMemcpyDeviceToHost, s));
     DQ_CUDA(cudaStreamSynchronize(s));
     if (*h_over > 65535) { g_err = "an instance leaves more than 65535 edges outside its neighbour rows"; return DQ_ERR_UNSUPPORTED; }
     A.over_cap = (int)((*h_over + 1) & ~1ull);
@@ -1488,10 +1482,7 @@ static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphB
     bool lane_engine = k <= 4 && (engine == DQ_ENGINE_LANE || (engine == DQ_ENGINE_AUTO && n >= 4096));
     DevBuf<uint32_t> d_ent_off, d_ent; DevBuf<uint8_t> d_adj;
     DevBuf<unsigned long long> d_ctrl;
-    struct Guard {                                       // buffers go back to the block cache only after the queue has drained
-        cudaStream_t s; DevBuf<uint32_t>&a, &b; DevBuf<uint8_t>& c; DevBuf<unsigned long long>& d;
-        ~Guard() { cudaStreamSynchronize(s); a.release(); b.release(); c.release(); d.release(); }
-    } guard{s, d_ent_off, d_ent, d_adj, d_ctrl};
+    StreamDrain drain{s};
     DQ_CUDA(d_ctrl.reserve(8));
     DQ_CUDA(cudaMemsetAsync(d_ctrl.p, 0, 8 * sizeof(unsigned long long), s));
     unsigned long long launches = 0;
@@ -1548,8 +1539,8 @@ static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphB
     }
     DQ_CUDA(cudaGetLastError());
     DQ_CUDA(cudaEventRecord(ctx->ev1, s));
-    unsigned long long* h = ctx->pin + 128 - 8;          // (pinned: the copy is asynchronous)
-    DQ_CUDA(cudaMemcpyAsync(h, d_ctrl.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    unsigned long long* h = ctx->pin->graphs_ctrl;
+    DQ_CUDA(cudaMemcpyAsync(h, d_ctrl.p, sizeof ctx->pin->graphs_ctrl, cudaMemcpyDeviceToHost, s));
     DQ_CUDA(cudaStreamSynchronize(s));
     DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     DQ_CUDA(cudaEventElapsedTime(&ms_search, ctx->ev2, ctx->ev3));
@@ -1593,10 +1584,7 @@ int dq_solve_batch_graphs(int32_t nv, int32_t k, const int64_t* edge_off, const 
     DQ_CUDA(device_ctx(&ctx));
     cudaStream_t s = ctx->stream;
     DevBuf<long long> d_off; DevBuf<uint8_t> d_edges, d_col, d_status; DevBuf<unsigned long long> d_nodes;
-    struct Guard {
-        cudaStream_t s; DevBuf<long long>& a; DevBuf<uint8_t>&b, &c, &d; DevBuf<unsigned long long>& e;
-        ~Guard() { cudaStreamSynchronize(s); a.release(); b.release(); c.release(); d.release(); e.release(); }
-    } guard{s, d_off, d_edges, d_col, d_status, d_nodes};
+    StreamDrain drain{s};
     const long long edge_bytes = (2 * total + 15) & ~15ll;
     DQ_CUDA(d_off.reserve(n + 1)); DQ_CUDA(d_edges.reserve(std::max<long long>(edge_bytes, 16))); DQ_CUDA(d_col.reserve((size_t)n * nv));
     DQ_CUDA(d_status.reserve(n)); DQ_CUDA(d_nodes.reserve(n));
