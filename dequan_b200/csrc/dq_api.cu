@@ -1217,7 +1217,8 @@ static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int
     BatchCellsArgs A;
     A.idx_list = idx_list;
     A.cells = cells_dev; A.n = n; A.stride = stride; A.cell_lut = m->t_cell_lut; A.values = m->t_values;
-    A.sizes = m->t_sizes; A.n_sizes = m->n_sizes; A.budget = opts ? opts->node_budget : 0;
+    A.sizes = m->t_sizes; A.n_sizes = m->n_sizes; A.caller_order = m->cm.caller_order ? 1 : 0;
+    A.budget = opts ? opts->node_budget : 0;
     A.cursor = ctrl; A.solution = sol_dev; A.nodes = nodes_dev; A.status = status_dev; A.totals = ctrl + 1;
     long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)occ * ctx->sm_count);
     if (ctas < 1) ctas = 1;
@@ -1529,7 +1530,7 @@ static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphB
             if (rc != DQ_OK) return rc;
             DQ_CUDA(d_ent_off.reserve((size_t)n * (nv + 1))); DQ_CUDA(d_ent.reserve(2 * (size_t)std::max<long long>(total, 1)));
             A.ent_off = d_ent_off.p; A.ent = d_ent.p;
-            k_graphs_build<<<(unsigned)((n + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, (size_t)kWarpsPerCta * (nv + 1) * 4, s>>>(A);
+            k_graphs_build<<<(unsigned)((n + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, kWarpsPerCta * graphs_build_warp_bytes(nv), s>>>(A);
             long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)std::max(occ, 1) * sms);
             DQ_CUDA(cudaEventRecord(ctx->ev2, s));
             k_batch_graphs<<<(unsigned)ctas, kWarpsPerCta * 32, smem, s>>>(A);

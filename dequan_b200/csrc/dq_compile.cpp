@@ -138,6 +138,7 @@ int compile_model(const dq_model_desc* d, CompiledModel& M, std::string& err) {
             seen[v] = 1;
             M.order[p] = v;
         }
+        M.caller_order = true;
     }
     M.pos_of.resize(nv);
     for (int p = 0; p < nv; p++) M.pos_of[M.order[p]] = p;

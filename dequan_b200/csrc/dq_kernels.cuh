@@ -304,6 +304,7 @@ struct BatchCellsArgs {
     const int32_t* values;      // [nv][32] value index -> value
     const int32_t* sizes;       // distinct domain sizes after overrides, ascending
     int n_sizes;
+    int caller_order;           // the template's assign_order came from the caller: every instance searches in it
     unsigned long long budget;
     unsigned long long* cursor;
     uint8_t* solution;          // [n][stride]
@@ -348,16 +349,21 @@ k_batch_cells(TreeModelDev M, BatchCellsArgs A) {
         }
         bad = __any_sync(FULL, bad);
         __syncwarp();
-        // static order for THIS instance: (domain size asc, id asc) — Assignment::Reset, dequan.h:384-394
-        int base = 0;
-        for (int s = 0; s < A.n_sizes; s++) {
-            const int sz = __ldg(A.sizes + s);
-            for (int v0 = 0; v0 < nv; v0 += 32) {
-                const int v = v0 + lane;
-                const bool hit = v < nv && __popc(S.D[v]) == sz;
-                const uint32_t m = __ballot_sync(FULL, hit);
-                if (hit) { const int p = base + __popc(m & lt); S.order[p] = (uint16_t)v; S.pos[v] = (uint16_t)p; }
-                base += __popc(m);
+        if (A.caller_order) {
+            // a caller-supplied assign_order replaces Reset's sort (dequan.h:316), givens or not
+            for (int v = lane; v < nv; v += 32) { S.order[v] = __ldg(M.order + v); S.pos[v] = __ldg(M.pos + v); }
+        } else {
+            // static order for THIS instance: (domain size asc, id asc) — Assignment::Reset, dequan.h:384-394
+            int base = 0;
+            for (int s = 0; s < A.n_sizes; s++) {
+                const int sz = __ldg(A.sizes + s);
+                for (int v0 = 0; v0 < nv; v0 += 32) {
+                    const int v = v0 + lane;
+                    const bool hit = v < nv && __popc(S.D[v]) == sz;
+                    const uint32_t m = __ballot_sync(FULL, hit);
+                    if (hit) { const int p = base + __popc(m & lt); S.order[p] = (uint16_t)v; S.pos[v] = (uint16_t)p; }
+                    base += __popc(m);
+                }
             }
         }
         __syncwarp();
@@ -397,19 +403,34 @@ struct BatchGraphsArgs {
     int trail;
 };
 
+// k_graphs_build's shared memory per warp: deg[nv + 1] and an nv x nv adjacency bit matrix
+__host__ __device__ inline size_t graphs_build_warp_bytes(int nv) { return ((size_t)(nv + 1) + (size_t)nv * ((nv + 31) / 32)) * 4; }
+
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 k_graphs_build(BatchGraphsArgs A) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const long long i = (long long)blockIdx.x * kWarpsPerCta + wib;
     if (i >= A.n) return;
-    uint32_t* deg = (uint32_t*)smem + (size_t)wib * (A.nv + 1);
+    const int nw = (A.nv + 31) / 32;
+    uint32_t* deg = (uint32_t*)(smem + (size_t)wib * graphs_build_warp_bytes(A.nv));
+    uint32_t* adj = deg + A.nv + 1;                   // row v: the neighbours of v
     const long long e0 = A.edge_off[i], e1 = A.edge_off[i + 1];
     for (int v = lane; v <= A.nv; v += 32) deg[v] = 0;
+    for (int w = lane; w < A.nv * nw; w += 32) adj[w] = 0;
     __syncwarp();
+    // A repeated or reversed edge is one neighbour: fc_apply trails every entry that changes a domain word, and two
+    // entries on the same neighbour in one 32-lane pass would both be trailed, past the trail's nv * k + 32 bound.
     for (long long e = e0 + lane; e < e1; e += 32) {
-        atomicAdd(&deg[A.edges[2 * e]], 1u);
-        atomicAdd(&deg[A.edges[2 * e + 1]], 1u);
+        const int u = A.edges[2 * e], v = A.edges[2 * e + 1];
+        atomicOr(&adj[u * nw + (v >> 5)], 1u << (v & 31));
+        atomicOr(&adj[v * nw + (u >> 5)], 1u << (u & 31));
+    }
+    __syncwarp();
+    for (int v = lane; v < A.nv; v += 32) {
+        uint32_t d = 0;
+        for (int w = 0; w < nw; w++) d += __popc(adj[v * nw + w]);
+        deg[v] = d;
     }
     __syncwarp();
     // exclusive scan of deg[0..nv) by the warp, 32 at a time
@@ -426,14 +447,13 @@ k_graphs_build(BatchGraphsArgs A) {
     if (lane == 0) off[A.nv] = carry;
     __syncwarp();
     uint32_t* ent = A.ent + 2 * e0;
-    // fill in edge order so that each adjacency list is deterministic: lane 0 walks the edges
-    // (a few hundred per instance; this kernel is <1% of the solve)
-    if (lane == 0)
-        for (long long e = e0; e < e1; e++) {
-            const int u = A.edges[2 * e], v = A.edges[2 * e + 1];
-            ent[deg[u]++] = (uint32_t)v | (D_K_NE_SAME << D_KIND_SHIFT);
-            ent[deg[v]++] = (uint32_t)u | (D_K_NE_SAME << D_KIND_SHIFT);
-        }
+    // each adjacency list in ascending neighbour id (deterministic; the order of a variable's entries changes no result)
+    for (int v = lane; v < A.nv; v += 32) {
+        uint32_t o = deg[v];
+        for (int w = 0; w < nw; w++)
+            for (uint32_t b = adj[v * nw + w]; b; b &= b - 1)
+                ent[o++] = (uint32_t)(w * 32 + __ffs((int)b) - 1) | (D_K_NE_SAME << D_KIND_SHIFT);
+    }
 }
 
 __global__ void __launch_bounds__(kWarpsPerCta * 32)

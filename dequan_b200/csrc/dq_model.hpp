@@ -58,8 +58,9 @@ struct CompiledModel {
     bool wide() const { return kmax > 32; }    // 64-bit domain words on the device (generic tree engine only)
     std::vector<std::vector<int32_t>> values;  // [nv][k_v]
     std::vector<Mask> dom0;                    // [nv] initial domain bits
-    std::vector<int32_t> order;                // [nv] position -> var id (Reset order)
+    std::vector<int32_t> order;                // [nv] position -> var id (Reset order, or the caller's assign_order)
     std::vector<int32_t> pos_of;               // [nv] var id -> position
+    bool caller_order = false;                 // `order` is the caller's assign_order: batches keep it for every instance
     std::vector<uint32_t> ent_off;             // [nv+1]
     std::vector<uint32_t> ent;                 // [n_ent]
     std::vector<uint32_t> ent_moff;            // [n_ent] index into masks (kinds != K_NE_SAME)

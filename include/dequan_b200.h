@@ -167,7 +167,8 @@ typedef struct dq_batch_opts {
 } dq_batch_opts;
 
 typedef struct dq_batch_stats {
-    uint64_t n_sat, n_unsat, n_budget;
+    uint64_t n_sat, n_unsat, n_budget;   /* n_sat + n_unsat + n_budget == n.  Status-3 rows (a given that is not
+                                            in its variable's template domain) count under n_unsat.          */
     uint64_t total_nodes;
     double   kernel_ms;
     uint64_t kernel_launches;
@@ -233,8 +234,11 @@ int dq_enumerate_solutions(dq_model *m, const dq_tree_opts *opts, dq_tree_result
 /* Batch of independent instances sharing the template's constraint graph but with
  * per-instance initial domains: cells[i*stride + v] == 0 keeps variable v's template
  * domain, any other byte c fixes it to the single value c (AddFixedVar, dequan.h:467).
- * Per instance: FIRST-mode solve; outputs status[i] (dq_outcome), nodes[i],
- * solution[i*stride + v] (value as byte, 0 if none).  Host buffers.               */
+ * Per instance: FIRST-mode solve; outputs status[i] (dq_outcome, or 3 with 0 nodes when a
+ * given byte is not a value of its variable's template domain), nodes[i],
+ * solution[i*stride + v] (value as byte, 0 if none).  Each instance is searched in
+ * Reset's order of its own domains, or in the template's assign_order if the caller
+ * supplied one.  Host buffers.                                                    */
 int dq_solve_batch_cells(dq_model *tmpl, const uint8_t *cells, int64_t n, int32_t stride,
                          const dq_batch_opts *opts, uint8_t *solution,
                          uint64_t *nodes, uint8_t *status, dq_batch_stats *stats);
