@@ -54,7 +54,7 @@ class dq_batch_stats(C.Structure):
 
 
 EXPORTS = ["dq_device_info", "dq_set_device", "dq_compile", "dq_free", "dq_model_info", "dq_model_order", "dq_model_table_bytes", "dq_solve_tree",
-           "dq_solve_tree_multi", "dq_tree_nodes_upto", "dq_enumerate_solutions", "dq_solve_batch_cells", "dq_solve_batch_cells_dev", "dq_solve_batch_graphs", "dq_solve_batch_graphs_dev",
+           "dq_solve_tree_multi", "dq_solve_models", "dq_tree_nodes_upto", "dq_enumerate_solutions", "dq_solve_batch_cells", "dq_solve_batch_cells_dev", "dq_solve_batch_graphs", "dq_solve_batch_graphs_dev",
            "dq_measure_int_peak", "dq_last_error", "dq_version", "dq_parse_sudoku_lines", "dq_parse_dimacs_col"]
 
 _lib = None
@@ -79,6 +79,8 @@ def lib():
     L.dq_model_table_bytes.argtypes = [vp, C.POINTER(C.c_uint64)]
     L.dq_solve_tree.argtypes = [vp, C.POINTER(dq_tree_opts), C.POINTER(dq_tree_result), i32p]
     L.dq_solve_tree_multi.argtypes = [vp, C.POINTER(dq_tree_opts), C.c_int32, i32p, C.POINTER(dq_tree_result), i32p]
+    L.dq_solve_models.argtypes = [C.POINTER(vp), C.c_int64, C.POINTER(dq_tree_opts), i32p, u64p, u64p, i32p,
+                                  C.POINTER(C.c_int64), C.POINTER(dq_batch_stats)]
     L.dq_tree_nodes_upto.argtypes = [vp, C.c_uint64, C.POINTER(C.c_uint64)]
     L.dq_enumerate_solutions.argtypes = [vp, C.POINTER(dq_tree_opts), C.POINTER(dq_tree_result), i32p, C.c_uint64, C.POINTER(C.c_uint64)]
     L.dq_solve_batch_cells.argtypes = [vp, u8p, C.c_int64, C.c_int32, C.POINTER(dq_batch_opts), u8p, u64p, u8p,
@@ -266,6 +268,43 @@ class Model:
         fn = lib().dq_solve_batch_cells_dev if device else lib().dq_solve_batch_cells
         _check(fn(self._h, cells_ptr, n, stride, C.byref(o), sol_ptr, nodes_ptr, status_ptr, C.byref(st)))
         return st
+
+
+@dataclass
+class ModelsResult:
+    """Per model, in list order, what `Model.solve_tree(mode)` reports: status, solutions, nodes, first."""
+    status: List[str]
+    solutions: List[int]
+    nodes: List[int]
+    first: List[Optional[List[int]]]
+    n_split: int
+    kernel_ms: float
+    launches: int
+
+
+def solve_models(models, mode: str = "first", engine: str = "auto") -> ModelsResult:
+    """dq_solve_models: many independent compiled models in one call.  `models` is a sequence of `Model` (the same one
+    may appear more than once; None passes a NULL handle)."""
+    n = len(models)
+    hs = (C.c_void_p * max(n, 1))(*[m._h.value if m is not None and m._h else None for m in models])
+    nvs = [m.n_vars if m is not None else 0 for m in models]
+    off = np.concatenate([[0], np.cumsum(nvs, dtype=np.int64)])
+    outcome = np.zeros(max(n, 1), dtype=np.int32)
+    sols = np.zeros(max(n, 1), dtype=np.uint64)
+    nodes = np.zeros(max(n, 1), dtype=np.uint64)
+    first = np.zeros(max(int(off[-1]), 1), dtype=np.int32)
+    n_split = C.c_int64()
+    o = dq_tree_opts(DQ_MODE_COUNT_ALL if mode == "count" else DQ_MODE_FIRST, 0, 0, 1, 0, ENGINE[engine], 0)
+    st = dq_batch_stats()
+    i32 = C.POINTER(C.c_int32)
+    _check(lib().dq_solve_models(hs, n, C.byref(o), outcome.ctypes.data_as(i32), sols.ctypes.data, nodes.ctypes.data,
+                                 first.ctypes.data_as(i32), C.byref(n_split), C.byref(st)))
+    firsts = []
+    for i in range(n):
+        f = first[off[i]:off[i + 1]].tolist()
+        firsts.append(f if sols[i] and (nvs[i] == 0 or f[0] != UNASSIGNED) else None)
+    return ModelsResult([OUTCOME[int(x)] for x in outcome[:n]], [int(x) for x in sols[:n]], [int(x) for x in nodes[:n]],
+                        firsts, n_split.value, st.kernel_ms, st.kernel_launches)
 
 
 def solve_batch_graphs(n_vertices: int, k: int, edge_off: np.ndarray, edges: np.ndarray, node_budget: int = 0,

@@ -247,21 +247,51 @@ struct dq_model {
 
 namespace dq {
 
+// A handle is bound to the device (and thread) of its first solve: its stream, events and cached blocks live there.
+static int check_bound(const dq_model* m, int dev) {
+    if (m->ctx && dev != m->ctx->dev) { g_err = "model handle is bound to CUDA device " + std::to_string(m->ctx->dev) + " (dq_set_device before the first solve)"; return DQ_ERR_INVALID; }
+    return DQ_OK;
+}
+
+// Appends one table to a host image at the next multiple of `align` bytes (at least 4 bytes, zero-filled).
+template <class V>
+static size_t put_table(std::vector<uint8_t>& blob, const V& vec, size_t align) {
+    const size_t off = (blob.size() + align - 1) & ~(align - 1);
+    blob.resize(off + std::max<size_t>(vec.size() * sizeof(vec[0]), 4), 0);
+    if (!vec.empty()) memcpy(blob.data() + off, vec.data(), vec.size() * sizeof(vec[0]));
+    return off;
+}
+
+// The generic tree engine's tables of one model, in this order: ent_off, ent, ent_moff, masks and dom0 (32-bit words, or
+// 64-bit when the model is wide), order and pos (16-bit).  upload() and dq_solve_models both pack them here.
+struct TreeTableOffsets { size_t ent_off, ent, ent_moff, masks, dom0, order, pos; };
+static TreeTableOffsets put_tree_tables(const CompiledModel& c, std::vector<uint8_t>& blob, size_t align) {
+    const int nv = c.nv;
+    std::vector<uint16_t> order(nv), pos(nv);
+    for (int i = 0; i < nv; i++) { order[i] = (uint16_t)c.order[i]; pos[i] = (uint16_t)c.pos_of[i]; }
+    // domain words on the device: 32 bits unless some domain has more than 32 values
+    std::vector<uint32_t> masks32, dom032;
+    if (!c.wide()) { masks32.assign(c.masks.begin(), c.masks.end()); dom032.assign(c.dom0.begin(), c.dom0.end()); }
+    TreeTableOffsets o;
+    o.ent_off = put_table(blob, c.ent_off, align);
+    o.ent = put_table(blob, c.ent, align);
+    o.ent_moff = put_table(blob, c.ent_moff, align);
+    o.masks = c.wide() ? put_table(blob, c.masks, align) : put_table(blob, masks32, align);
+    o.dom0 = c.wide() ? put_table(blob, c.dom0, align) : put_table(blob, dom032, align);
+    o.order = put_table(blob, order, align);
+    o.pos = put_table(blob, pos, align);
+    return o;
+}
+
 static int upload(dq_model* m) {
     int dev = 0;
     DQ_CUDA(cudaGetDevice(&dev));
-    if (m->ctx) {
-        // a handle is bound to the device (and thread) of its first solve: its stream, events and cached blocks live there
-        if (dev != m->ctx->dev) { g_err = "model handle is bound to CUDA device " + std::to_string(m->ctx->dev) + " (dq_set_device before the first solve)"; return DQ_ERR_INVALID; }
-        return DQ_OK;
-    }
+    if (m->ctx) return check_bound(m, dev);
     DeviceCtx* ctx = nullptr;
     DQ_CUDA(device_ctx(&ctx));
     const CompiledModel& c = m->cm;
     const int nv = c.nv;
     // every table goes into ONE device block with ONE stream-ordered copy (the solve's kernels follow on the same stream)
-    std::vector<uint16_t> order(nv), pos(nv);
-    for (int i = 0; i < nv; i++) { order[i] = (uint16_t)c.order[i]; pos[i] = (uint16_t)c.pos_of[i]; }
     std::vector<int32_t> values((size_t)nv * 32, 0);
     std::vector<uint8_t> lut((size_t)nv * 256, 0xFF);
     for (int v = 0; v < nv; v++)
@@ -275,18 +305,9 @@ static int upload(dq_model* m) {
     m->n_sizes = (int)sizes.size();
     std::vector<uint8_t>& blob = m->h_blob;
     blob.clear();
-    auto put = [&](const auto& vec) -> size_t {
-        const size_t off = (blob.size() + 255) & ~(size_t)255;
-        blob.resize(off + std::max<size_t>(vec.size() * sizeof(vec[0]), 4), 0);
-        if (!vec.empty()) memcpy(blob.data() + off, vec.data(), vec.size() * sizeof(vec[0]));
-        return off;
-    };
-    // domain words on the device: 32 bits unless some domain has more than 32 values
-    std::vector<uint32_t> masks32, dom032;
-    if (!c.wide()) { masks32.assign(c.masks.begin(), c.masks.end()); dom032.assign(c.dom0.begin(), c.dom0.end()); }
-    const size_t o_ent_off = put(c.ent_off), o_ent = put(c.ent), o_ent_moff = put(c.ent_moff),
-                 o_masks = c.wide() ? put(c.masks) : put(masks32), o_dom0 = c.wide() ? put(c.dom0) : put(dom032), o_order = put(order), o_pos = put(pos), o_values = put(values), o_lut = put(lut),
-                 o_sizes = put(sizes);
+    auto put = [&](const auto& vec) -> size_t { return put_table(blob, vec, 256); };
+    const TreeTableOffsets t = put_tree_tables(c, blob, 256);
+    const size_t o_values = put(values), o_lut = put(lut), o_sizes = put(sizes);
     std::vector<uint32_t> dom0_pos(32, 0xFFFFFFFFu);
     for (int p = 0; p < nv && p < 32; p++) dom0_pos[p] = (uint32_t)c.dom0[c.order[p]];
     const size_t o_s_and = put(c.small_and), o_s_weq = put(c.small_weq), o_s_weq_on = put(c.small_weq_on), o_s_chk = put(c.small_chk),
@@ -294,8 +315,8 @@ static int upload(dq_model* m) {
     DQ_CUDA(m->d_blob.reserve(blob.size()));
     DQ_CUDA(cudaMemcpyAsync(m->d_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice, ctx->stream));
     uint8_t* base = m->d_blob.p;
-    m->t_ent_off = (uint32_t*)(base + o_ent_off); m->t_ent = (uint32_t*)(base + o_ent); m->t_ent_moff = (uint32_t*)(base + o_ent_moff);
-    m->t_masks = (uint32_t*)(base + o_masks); m->t_dom0 = (uint32_t*)(base + o_dom0); m->t_order = (uint16_t*)(base + o_order); m->t_pos = (uint16_t*)(base + o_pos);
+    m->t_ent_off = (uint32_t*)(base + t.ent_off); m->t_ent = (uint32_t*)(base + t.ent); m->t_ent_moff = (uint32_t*)(base + t.ent_moff);
+    m->t_masks = (uint32_t*)(base + t.masks); m->t_dom0 = (uint32_t*)(base + t.dom0); m->t_order = (uint16_t*)(base + t.order); m->t_pos = (uint16_t*)(base + t.pos);
     m->t_values = (int32_t*)(base + o_values); m->t_cell_lut = base + o_lut; m->t_sizes = (int32_t*)(base + o_sizes);
     m->t_s_and = (uint32_t*)(base + o_s_and); m->t_s_weq = (uint32_t*)(base + o_s_weq); m->t_s_weq_on = (uint32_t*)(base + o_s_weq_on);
     m->t_s_chk = (uint32_t*)(base + o_s_chk); m->t_s_dom0 = (uint32_t*)(base + o_s_dom0);
@@ -335,10 +356,12 @@ template <> struct LevelWords<W64> {
 // Calls f(has_f, has_table) with the model's feature flags as std::bool_constant, so that f can name the kernel
 // instantiation for them: with_features(m->cm, [&](auto hf, auto ht) { k<hf, ht><<<...>>>(...); }).
 template <class F>
-static auto with_features(const CompiledModel& cm, F&& f) {
-    if (cm.has_f) return cm.has_table ? f(std::true_type{}, std::true_type{}) : f(std::true_type{}, std::false_type{});
-    return cm.has_table ? f(std::false_type{}, std::true_type{}) : f(std::false_type{}, std::false_type{});
+static auto with_features(bool has_f, bool has_table, F&& f) {
+    if (has_f) return has_table ? f(std::true_type{}, std::true_type{}) : f(std::true_type{}, std::false_type{});
+    return has_table ? f(std::false_type{}, std::true_type{}) : f(std::false_type{}, std::false_type{});
 }
+template <class F>
+static auto with_features(const CompiledModel& cm, F&& f) { return with_features(cm.has_f, cm.has_table, std::forward<F>(f)); }
 
 template <class K>
 static int max_ctas_per_sm(K kernel, int threads, size_t smem, int* out) {
@@ -1188,6 +1211,181 @@ int dq_solve_tree_multi(dq_model* m, const dq_tree_opts* opts, int32_t n_devices
     res->outcome = res->n_solutions ? DQ_SAT : DQ_UNSAT;
     if (first_solution)
         for (int v = 0; v < nv; v++) first_solution[v] = key != KEY_NONE ? mc->w[owner]->first[v] : -2147483647;
+    return DQ_OK;
+}
+
+}  // extern "C" (templates follow)
+
+// ---- many independent models in one call (dq_solve_models) ----
+// The models' generic tables are packed into one host image behind the slot records and the launch cursors, and go to
+// the device in one copy.  Launches are grouped by domain word and by state size class (warp_state_bytes rounded up to a
+// power of two), so that one large model does not cut the occupancy of many small ones.  Each warp takes whole models
+// from its launch's cursor and searches each under kModelWarpNodes; a model past that budget is marked split and solved
+// afterwards by solve_tree_impl, so every answer is what dq_solve_tree gives for that handle.
+struct ModelsGroup {
+    bool wide, has_f, has_table;
+    size_t warp_bytes;             // the largest state of the group
+    int wpc;                       // warps per CTA
+    long long s0, s1;              // its slots
+};
+
+template <typename W>
+static int launch_models(const ModelsGroup& g, const ModelsArgs& A, DeviceCtx* ctx) {
+    const size_t smem = g.warp_bytes * g.wpc;
+    int occ = 0;
+    int rc = with_features(g.has_f, g.has_table, [&](auto hf, auto ht) { return max_ctas_per_sm(k_models_dfs<hf, ht, W>, g.wpc * 32, smem, &occ); });
+    if (rc != DQ_OK) return rc;
+    if (occ < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
+    const long long ctas = std::max<long long>(1, std::min<long long>((A.n + g.wpc - 1) / g.wpc, (long long)occ * ctx->sm_count));
+    with_features(g.has_f, g.has_table, [&](auto hf, auto ht) { k_models_dfs<hf, ht, W><<<(int)ctas, g.wpc * 32, smem, ctx->stream>>>(A); });
+    DQ_CUDA(cudaGetLastError());
+    return DQ_OK;
+}
+
+extern "C" {
+
+int dq_solve_models(dq_model* const* models, int64_t n, const dq_tree_opts* opts, int32_t* outcome, uint64_t* n_solutions,
+                    uint64_t* n_nodes, int32_t* solutions, int64_t* n_split, dq_batch_stats* stats) {
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (n_split) *n_split = 0;
+    if (n < 0 || !opts) { g_err = "bad argument"; return DQ_ERR_INVALID; }
+    if (opts->mode != DQ_MODE_FIRST && opts->mode != DQ_MODE_COUNT_ALL) { g_err = "bad mode"; return DQ_ERR_INVALID; }
+    if (opts->part_count < 1 || opts->part_rank < 0 || opts->part_rank >= opts->part_count) { g_err = "bad partition"; return DQ_ERR_INVALID; }
+    if (opts->part_count > 1) { g_err = "dq_solve_models solves whole trees: one partition"; return DQ_ERR_UNSUPPORTED; }
+    if (opts->split_depth > 0) { g_err = "dq_solve_models chooses the split itself: split_depth must be <= 0"; return DQ_ERR_UNSUPPORTED; }
+    if (opts->node_budget) { g_err = "node_budget is a batch option; single-tree solves have none"; return DQ_ERR_UNSUPPORTED; }
+    if (opts->engine != DQ_ENGINE_AUTO && opts->engine != DQ_ENGINE_WARP) { g_err = "dq_solve_models runs the generic warp engine: engine AUTO or WARP"; return DQ_ERR_UNSUPPORTED; }
+    if (n == 0) return DQ_OK;
+    if (!models || !outcome || !n_solutions || !n_nodes) { g_err = "null buffer"; return DQ_ERR_INVALID; }
+    for (int64_t i = 0; i < n; i++)
+        if (!models[i]) { g_err = "null model at index " + std::to_string(i); return DQ_ERR_INVALID; }
+    int dev = 0;
+    DQ_CUDA(cudaGetDevice(&dev));
+    for (int64_t i = 0; i < n; i++) {
+        const int rc = check_bound(models[i], dev);
+        if (rc != DQ_OK) return rc;
+    }
+    DeviceCtx* ctx = nullptr;
+    DQ_CUDA(device_ctx(&ctx));
+    const bool count_all = opts->mode == DQ_MODE_COUNT_ALL;
+    const int UNASSIGNED = -2147483647;
+    std::vector<int64_t> sol_off(n + 1, 0);                // each model's first value in `solutions`
+    for (int64_t i = 0; i < n; i++) sol_off[i + 1] = sol_off[i] + models[i]->cm.nv;
+
+    // slots in launch order: by domain word, then by state size class
+    std::vector<int64_t> idx;
+    std::vector<size_t> wbytes(n, 0);
+    for (int64_t i = 0; i < n; i++) {
+        const CompiledModel& c = models[i]->cm;
+        if (c.nv == 0) continue;
+        wbytes[i] = warp_state_bytes(c.nv, c.trail_bound, c.wide() ? 8 : 4);
+        idx.push_back(i);
+    }
+    auto size_class = [&](int64_t i) { size_t s = 16; while (s < wbytes[i]) s <<= 1; return s; };
+    std::stable_sort(idx.begin(), idx.end(), [&](int64_t a, int64_t b) {
+        const bool wa = models[a]->cm.wide(), wb = models[b]->cm.wide();
+        return wa != wb ? wb : size_class(a) < size_class(b);
+    });
+    const long long n_slots = (long long)idx.size();
+    std::vector<ModelsGroup> groups;
+    for (long long k = 0; k < n_slots; k++) {
+        const CompiledModel& c = models[idx[k]]->cm;
+        if (groups.empty() || groups.back().wide != c.wide() || size_class(idx[groups.back().s0]) != size_class(idx[k]))
+            groups.push_back(ModelsGroup{c.wide(), false, false, 0, 0, k, k});
+        ModelsGroup& g = groups.back();
+        g.has_f |= c.has_f; g.has_table |= c.has_table;
+        g.warp_bytes = std::max(g.warp_bytes, wbytes[idx[k]]);
+        g.s1 = k + 1;
+    }
+    for (ModelsGroup& g : groups) {
+        g.wpc = (int)std::min<size_t>(kWarpsPerCta, (200 * 1024) / g.warp_bytes);
+        if (g.wpc < 1) { g_err = "model state exceeds shared memory"; return DQ_ERR_UNSUPPORTED; }
+    }
+
+    // host image: launch cursors, slot records, then every model's tables
+    const size_t o_slots = ((groups.size() * 8 + 15) & ~(size_t)15);
+    std::vector<uint8_t> blob(o_slots + (size_t)n_slots * sizeof(ModelSlot), 0);
+    std::vector<ModelSlot> slots(n_slots);
+    unsigned long long sol_bytes = 0;
+    for (long long k = 0; k < n_slots; k++) {
+        const CompiledModel& c = models[idx[k]]->cm;
+        const TreeTableOffsets t = put_tree_tables(c, blob, 16);
+        ModelSlot& s = slots[k];
+        s.base = t.ent_off;
+        s.o_ent = (uint32_t)(t.ent - t.ent_off); s.o_ent_moff = (uint32_t)(t.ent_moff - t.ent_off);
+        s.o_masks = (uint32_t)(t.masks - t.ent_off); s.o_dom0 = (uint32_t)(t.dom0 - t.ent_off);
+        s.o_order = (uint32_t)(t.order - t.ent_off); s.o_pos = (uint32_t)(t.pos - t.ent_off);
+        s.nv = c.nv; s.trail = c.trail_bound;
+        s.sol = sol_bytes;
+        sol_bytes += (unsigned long long)c.nv;
+    }
+    if (n_slots) memcpy(blob.data() + o_slots, slots.data(), slots.size() * sizeof(ModelSlot));
+
+    // results: one record per slot, then the value indices of every slot's first solution
+    const size_t o_sol = (size_t)n_slots * sizeof(ModelOut);
+    const size_t read_bytes = o_sol + (solutions ? (size_t)sol_bytes : 0);
+    std::vector<uint8_t> h_out(read_bytes);
+    DevBuf<uint8_t> d_in, d_out;
+    StreamDrain drain{ctx->stream};
+    float ms = 0;
+    unsigned long long launches = 0;
+    if (n_slots) {
+        DQ_CUDA(d_in.reserve(blob.size()));
+        DQ_CUDA(d_out.reserve(o_sol + (size_t)sol_bytes));
+        DQ_CUDA(cudaMemcpyAsync(d_in.p, blob.data(), blob.size(), cudaMemcpyHostToDevice, ctx->stream));
+        DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+        for (size_t gi = 0; gi < groups.size(); gi++) {
+            const ModelsGroup& g = groups[gi];
+            ModelsArgs A;
+            A.slots = reinterpret_cast<const ModelSlot*>(d_in.p + o_slots) + g.s0;
+            A.n = g.s1 - g.s0;
+            A.tables = d_in.p;
+            A.warp_bytes = g.warp_bytes;
+            A.count_all = count_all ? 1 : 0;
+            A.cursor = reinterpret_cast<unsigned long long*>(d_in.p) + gi;
+            A.out = reinterpret_cast<ModelOut*>(d_out.p) + g.s0;
+            A.sol = d_out.p + o_sol;
+            const int rc = g.wide ? launch_models<W64>(g, A, ctx) : launch_models<uint32_t>(g, A, ctx);
+            if (rc != DQ_OK) return rc;
+            launches++;
+        }
+        DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+        DQ_CUDA(cudaMemcpyAsync(h_out.data(), d_out.p, read_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        DQ_CUDA(cudaStreamSynchronize(ctx->stream));
+        DQ_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    }
+
+    unsigned long long n_sat = 0, total_nodes = 0;
+    int64_t splits = 0;
+    for (int64_t i = 0; i < n; i++)
+        if (models[i]->cm.nv == 0) { outcome[i] = DQ_SAT; n_solutions[i] = 1; n_nodes[i] = 0; }      // IsComplete at entry
+    for (long long k = 0; k < n_slots; k++) {
+        const int64_t i = idx[k];
+        ModelOut o;
+        memcpy(&o, h_out.data() + (size_t)k * sizeof(ModelOut), sizeof o);
+        const CompiledModel& c = models[i]->cm;
+        if (o.outcome == DQ_BUDGET) {                       // past the warp's budget: the split search, as dq_solve_tree runs it
+            dq_tree_result r;
+            const int rc = solve_tree_impl(models[i], opts, &r, solutions ? solutions + sol_off[i] : nullptr, nullptr);
+            if (rc != DQ_OK) return rc;
+            outcome[i] = r.outcome; n_solutions[i] = r.n_solutions; n_nodes[i] = r.n_nodes;
+            launches += r.kernel_launches;
+            splits++;
+            continue;
+        }
+        outcome[i] = o.outcome; n_solutions[i] = o.sols; n_nodes[i] = o.nodes;
+        if (solutions) {
+            const uint8_t* v = h_out.data() + o_sol + slots[k].sol;
+            for (int x = 0; x < c.nv; x++) solutions[sol_off[i] + x] = o.sols ? c.values[x][v[x]] : UNASSIGNED;
+        }
+    }
+    for (int64_t i = 0; i < n; i++) { n_sat += outcome[i] == DQ_SAT; total_nodes += n_nodes[i]; }
+    if (n_split) *n_split = splits;
+    if (stats) {
+        stats->n_sat = n_sat; stats->n_unsat = (uint64_t)n - n_sat; stats->n_budget = 0; stats->total_nodes = total_nodes;
+        stats->kernel_ms = ms; stats->kernel_launches = launches;
+        stats->h2d_bytes = n_slots ? blob.size() : 0; stats->d2h_bytes = n_slots ? read_bytes : 0;
+    }
     return DQ_OK;
 }
 

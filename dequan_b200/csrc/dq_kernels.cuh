@@ -491,6 +491,81 @@ k_batch_graphs(BatchGraphsArgs A) {
     }
 }
 
+// ---- many independent models (dq_solve_models): one warp owns one model's whole tree -----------------------------
+// Node budget of one model inside the batch: a tree that is not finished by then is marked split and solved afterwards
+// by the single-model path.  Not yet measured: scripts/models_budget_sweep.py is the sweep that is to choose it
+// (DESIGN.md §4.1f).
+constexpr unsigned long long kModelWarpNodes = 1ull << 14;
+
+// Where one model's tables sit in the packed block (byte offsets from `base`; ent_off at `base` itself) and its slice of
+// the output value-index bytes.
+struct ModelSlot {
+    unsigned long long base;
+    uint32_t o_ent, o_ent_moff, o_masks, o_dom0, o_order, o_pos;
+    int nv, trail;
+    unsigned long long sol;
+};
+struct ModelOut {
+    unsigned long long nodes, sols;
+    int outcome;            // dq_outcome; DQ_BUDGET = split
+    int pad;
+};
+struct ModelsArgs {
+    const ModelSlot* slots;         // this launch's slots
+    long long n;
+    const uint8_t* tables;          // the packed block
+    size_t warp_bytes;              // shared memory per warp: the largest state of this launch
+    int count_all;
+    unsigned long long* cursor;
+    ModelOut* out;                  // [n] this launch's results
+    uint8_t* sol;                   // value index per var id, every model's slice
+};
+
+// The first solution of one model into its slice, value indices by var id.  Only this warp writes the slice.
+struct FirstToSlice {
+    uint8_t* dst;
+    int nv, lane;
+    template <typename W>
+    __device__ void operator()(const WarpStateT<W>& S) const {
+        for (int i = lane; i < nv; i += 32) dst[S.order[i]] = S.val[i];
+    }
+    template <typename W>
+    __device__ void solutions(const WarpStateT<W>&, W, unsigned long long) const {}
+};
+
+template <bool HAS_F, bool HAS_TABLE, typename W>
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+k_models_dfs(ModelsArgs A) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    unsigned char* region = smem + (size_t)wib * A.warp_bytes;
+    for (;;) {
+        long long j = 0;
+        if (lane == 0) j = (long long)atomicAdd(A.cursor, 1ull);
+        j = __shfl_sync(FULL, j, 0);
+        if (j >= A.n) break;
+        const ModelSlot s = A.slots[j];
+        const uint8_t* b = A.tables + s.base;
+        TreeModelDevT<W> M;
+        M.T.nv = s.nv;
+        M.T.ent_off = reinterpret_cast<const uint32_t*>(b);
+        M.T.ent = reinterpret_cast<const uint32_t*>(b + s.o_ent);
+        M.T.ent_moff = reinterpret_cast<const uint32_t*>(b + s.o_ent_moff);
+        M.T.masks = reinterpret_cast<const W*>(b + s.o_masks);
+        M.dom0 = reinterpret_cast<const W*>(b + s.o_dom0);
+        M.order = reinterpret_cast<const uint16_t*>(b + s.o_order);
+        M.pos = reinterpret_cast<const uint16_t*>(b + s.o_pos);
+        M.trail = s.trail;
+        const WarpStateT<W> S = carve_warp_state_t<W>(region, s.nv, s.trail);
+        load_root_state(M, S, lane);
+        const FirstToSlice rec{A.sol + s.sol, s.nv, lane};
+        const DfsResult R = warp_dfs<HAS_F, HAS_TABLE>(M.T, S, 0, A.count_all != 0, kModelWarpNodes, nullptr, 0ull, lane, rec);
+        if (!A.count_all && R.have_first) rec(S);
+        if (lane == 0) { A.out[j].nodes = R.nodes; A.out[j].sols = R.sols; A.out[j].outcome = R.outcome; }
+        __syncwarp();
+    }
+}
+
 // ---- integer-pipe peak: 8 independent lop3.b32 chains per lane, one LOP3 per statement ------------
 #define DQ_LOP3(d, a, b) asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(d) : "r"(a), "r"(b))
 __global__ void __launch_bounds__(1024) k_int_peak(uint32_t* out, int iters) {

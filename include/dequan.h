@@ -531,6 +531,13 @@ struct ModelCache {
     }
 };
 
+/* Many (CSP, Assignment) pairs in one device call (dq_solve_models).  Element i is what csps[i]->ForwardCheckingStep(*as[i])
+ * returns, and every Assignment is left exactly as that call leaves it.  Several pairs may share one CSP.  reps (may be
+ * null) is resized to the number of pairs; its tree results carry outcome, n_solutions and n_nodes, first_key only as a
+ * flag (0: a solution, UINT64_MAX: none; the batch reports no prefix keys), and every other field 0. */
+inline std::vector<bool> SolveAll(const std::vector<const CSP*>& csps, const std::vector<Assignment*>& as,
+                                  std::vector<SolveReport>* reps = nullptr);
+
 }  // namespace b200
 
 /* The model (reference dequan.h:328-355).  Static during the search. */
@@ -584,7 +591,18 @@ public:
                        std::vector<std::vector<int> >& out, unsigned long long max_solutions) const;
 
 private:
+    friend std::vector<bool> b200::SolveAll(const std::vector<const CSP*>&, const std::vector<Assignment*>&,
+                                            std::vector<b200::SolveReport>*);
+    /* The flattened descriptor of a lowering; `key` holds all of it in one flat vector (equal key: equal tables). */
+    struct Lowered {
+        b200::Lowering low;
+        std::vector<int32_t> dom_type, dom_off, dom_vals, order, key;
+    };
+    void Lower(const Assignment& a, Lowered& out) const;
+    static dq_model* Compile(const Lowered& l, int nv);
     bool CompileB200(const Assignment& a) const;
+    int CheckResumable(const Assignment& a) const;
+    bool FinishB200(Assignment& a, uint64_t nodes, bool have, const int32_t* first, int resumed) const;
     void Flatten(const Assignment& a, b200::Lowering& low, std::vector<int32_t>& dom_type, std::vector<int32_t>& dom_off,
                  std::vector<int32_t>& dom_vals) const;
     void TabulateUserConstraint(size_t c, b200::Lowering& low, const Assignment& a) const;
@@ -793,51 +811,96 @@ inline void CSP::Flatten(const Assignment& a, b200::Lowering& low, std::vector<i
     }
 }
 
+/* Lowers the CSP with the Assignment's domains and order. */
+inline void CSP::Lower(const Assignment& a, Lowered& l) const {
+    l.order.assign(a.assign_order.begin(), a.assign_order.end());
+    Flatten(a, l.low, l.dom_type, l.dom_off, l.dom_vals);
+    // one flat key for the cache: identical descriptor -> identical device tables
+    l.key.clear();
+    l.key.reserve(l.dom_type.size() + l.dom_off.size() + l.dom_vals.size() + l.order.size() + l.low.con_kind.size() +
+                  l.low.con_off.size() + l.low.con_data.size() + 8);
+    for (const std::vector<int32_t>* part : {&l.dom_type, &l.dom_off, &l.dom_vals, &l.order, &l.low.con_kind, &l.low.con_off, &l.low.con_data}) {
+        l.key.push_back((int32_t)part->size());
+        l.key.insert(l.key.end(), part->begin(), part->end());
+    }
+}
+
+inline dq_model* CSP::Compile(const Lowered& l, int nv) {
+    const int32_t zero = 0;
+    dq_model_desc desc{};
+    desc.n_vars = nv;
+    desc.dom_type = l.dom_type.empty() ? &zero : l.dom_type.data();
+    desc.dom_off = l.dom_off.data();
+    desc.dom_vals = l.dom_vals.empty() ? &zero : l.dom_vals.data();
+    desc.n_cons = (int32_t)l.low.con_kind.size();
+    desc.con_kind = l.low.con_kind.empty() ? &zero : l.low.con_kind.data();
+    desc.con_off = l.low.con_off.data();
+    desc.con_data = l.low.con_data.empty() ? &zero : l.low.con_data.data();
+    desc.assign_order = l.order.empty() ? nullptr : l.order.data();
+    dq_model* h = nullptr;
+    const int rc = dq_compile(&desc, &h);
+    if (rc != DQ_OK) throw b200::Error(rc, dq_last_error());
+    return h;
+}
+
 /* Lowers the CSP with the Assignment's domains and order and compiles it, unless the cached handle was built from the
  * identical descriptor.  Returns whether it compiled afresh. */
 inline bool CSP::CompileB200(const Assignment& a) const {
-    const int nv = (int)vars.size();
-    b200::Lowering low;
-    std::vector<int32_t> dom_type, dom_off, dom_vals, order(a.assign_order.begin(), a.assign_order.end());
-    Flatten(a, low, dom_type, dom_off, dom_vals);
-
-    // one flat key for the cache: identical descriptor -> identical device tables
-    std::vector<int32_t> key;
-    key.reserve(dom_type.size() + dom_off.size() + dom_vals.size() + order.size() + low.con_kind.size() + low.con_off.size() + low.con_data.size() + 8);
-    for (const std::vector<int32_t>* part : {&dom_type, &dom_off, &dom_vals, &order, &low.con_kind, &low.con_off, &low.con_data}) {
-        key.push_back((int32_t)part->size());
-        key.insert(key.end(), part->begin(), part->end());
-    }
-    const bool fresh = !cache_.handle || cache_.key != key;
+    Lowered l;
+    Lower(a, l);
+    const bool fresh = !cache_.handle || cache_.key != l.key;
     if (fresh) {
         cache_.Drop();
-        const int32_t zero = 0;
-        dq_model_desc desc{};
-        desc.n_vars = nv;
-        desc.dom_type = dom_type.empty() ? &zero : dom_type.data();
-        desc.dom_off = dom_off.data();
-        desc.dom_vals = dom_vals.empty() ? &zero : dom_vals.data();
-        desc.n_cons = (int32_t)low.con_kind.size();
-        desc.con_kind = low.con_kind.empty() ? &zero : low.con_kind.data();
-        desc.con_off = low.con_off.data();
-        desc.con_data = low.con_data.empty() ? &zero : low.con_data.data();
-        desc.assign_order = order.empty() ? nullptr : order.data();
-        const int rc = dq_compile(&desc, &cache_.handle);
-        if (rc != DQ_OK) throw b200::Error(rc, dq_last_error());
-        cache_.key.swap(key);
+        cache_.handle = Compile(l, (int)vars.size());
+        cache_.key.swap(l.key);
     }
     return fresh;
 }
 
-inline bool CSP::SolveB200(Assignment& a, int mode, const b200::SolveOptions& opt, b200::SolveReport* rep) const {
+/* Checks that `a` belongs to this CSP and that its assigned variables are a prefix of assign_order; returns the prefix's
+ * length (the reference resumes after it, dequan.h:504). */
+inline int CSP::CheckResumable(const Assignment& a) const {
     const int nv = (int)vars.size();
     if ((int)a.inst_vars.size() != nv || (int)a.current_domains.size() != nv || (int)a.assign_order.size() != nv)
         throw b200::Error(DQ_ERR_INVALID, "Assignment does not belong to this CSP: call a.Reset(csp) first");
-    const int resumed = a.assigned_var_count;            // a prefix of assign_order the caller assigned by hand (dequan.h:504)
+    const int resumed = a.assigned_var_count;
     for (int i = 0; i < nv; i++)
         if ((a.inst_vars[a.assign_order[i]].value != InstVar::UNASSIGNED) != (i < resumed))
             throw b200::Error(DQ_ERR_UNSUPPORTED, "the assigned variables must be the first assigned_var_count entries of assign_order");
+    return resumed;
+}
 
+/* Writes a device answer back into `a`: `nodes` is the device's node count (it visits each of the `resumed` pre-assigned
+ * singletons once; the reference does not), `first` the solution by var id when `have`.  Returns `have`. */
+inline bool CSP::FinishB200(Assignment& a, uint64_t nodes, bool have, const int32_t* first, int resumed) const {
+#ifdef DEQUAN_WITH_STATS
+    a.stats.assigned_vars += nodes - (uint64_t)resumed;
+#else
+    (void)nodes;
+#endif
+    if (!have) return false;
+    // Leave the Assignment as the reference's recursion leaves it on success: walk the one solution
+    // path, one saved-domain frame per depth, each linked constraint filtering in link order.
+    const int nv = (int)vars.size();
+    for (int d = resumed; d < nv; d++) {
+        const VarId vid = a.assign_order[d];
+        a.saved_domains.emplace_back();
+        a.inst_vars[vid].value = first[vid];
+        ++a.assigned_var_count;
+#ifdef DEQUAN_WITH_STATS
+        Stats keep = a.stats;
+#endif
+        for (Constraint* c : vars[vid].linked_constraints) c->AplyArcConsistency(a, vid);
+#ifdef DEQUAN_WITH_STATS
+        a.stats = keep;                              // applied_arcs is not reproduced (sequential early-exit dependent)
+#endif
+    }
+    return true;
+}
+
+inline bool CSP::SolveB200(Assignment& a, int mode, const b200::SolveOptions& opt, b200::SolveReport* rep) const {
+    const int nv = (int)vars.size();
+    const int resumed = CheckResumable(a);
     const bool fresh = CompileB200(a);
 
     dq_tree_opts o{};
@@ -853,28 +916,8 @@ inline bool CSP::SolveB200(Assignment& a, int mode, const b200::SolveOptions& op
     if (rc != DQ_OK) throw b200::Error(rc, dq_last_error());
     if (rep) { rep->tree = r; rep->compiled_fresh = fresh; }
     if (rep) rep->tree.n_nodes -= (uint64_t)resumed;     // (the device visits each pre-assigned singleton once; the reference does not)
-#ifdef DEQUAN_WITH_STATS
-    a.stats.assigned_vars += r.n_nodes - (uint64_t)resumed;
-#endif
     const bool have = r.first_key != UINT64_MAX && (nv == 0 || first[0] != InstVar::UNASSIGNED);
-    if (!have) return false;
-
-    // Leave the Assignment as the reference's recursion leaves it on success: walk the one solution
-    // path, one saved-domain frame per depth, each linked constraint filtering in link order.
-    for (int d = resumed; d < nv; d++) {
-        const VarId vid = a.assign_order[d];
-        a.saved_domains.emplace_back();
-        a.inst_vars[vid].value = first[vid];
-        ++a.assigned_var_count;
-#ifdef DEQUAN_WITH_STATS
-        Stats keep = a.stats;
-#endif
-        for (Constraint* c : vars[vid].linked_constraints) c->AplyArcConsistency(a, vid);
-#ifdef DEQUAN_WITH_STATS
-        a.stats = keep;                              // applied_arcs is not reproduced (sequential early-exit dependent)
-#endif
-    }
-    return true;
+    return FinishB200(a, r.n_nodes, have, first.data(), resumed);
 }
 
 inline void CSP::EnumerateB200(const Assignment& a, const b200::SolveOptions& opt, b200::SolveReport* rep,
@@ -943,6 +986,85 @@ inline void EnumerateAll(const CSP& csp, const Assignment& a, std::vector<std::v
                          unsigned long long max_solutions = 1000000ULL, const SolveOptions& opt = SolveOptions(),
                          SolveReport* rep = nullptr) {
     csp.EnumerateB200(a, opt, rep, out, max_solutions);
+}
+
+/* Complete Assignments answer true without a device call; the others go to the device in one dq_solve_models call.  A
+ * pair whose descriptor equals its CSP's cached one uses the cached handle; the first other descriptor of a CSP whose
+ * cache no earlier pair uses replaces the cache; any further one gets a handle that lives for this call only. */
+inline std::vector<bool> SolveAll(const std::vector<const CSP*>& csps, const std::vector<Assignment*>& as,
+                                  std::vector<SolveReport>* reps) {
+    if (csps.size() != as.size()) throw Error(DQ_ERR_INVALID, "SolveAll takes one Assignment per CSP");
+    const size_t n = csps.size();
+    std::vector<bool> out(n, false);
+    if (reps) reps->assign(n, SolveReport());
+    struct CallHandles {
+        std::vector<dq_model*> h;
+        ~CallHandles() { for (dq_model* p : h) dq_free(p); }
+    } call_handles;
+    struct Seen { const CSP* csp; std::vector<int32_t> key; dq_model* h; };
+    std::vector<Seen> seen;                                   // descriptors given a handle in this call
+    std::vector<size_t> todo;
+    std::vector<dq_model*> handles;
+    std::vector<int> resumed;
+    std::vector<char> fresh;
+    std::vector<size_t> off(1, 0);
+    for (size_t i = 0; i < n; i++) {
+        const CSP& csp = *csps[i];
+        Assignment& a = *as[i];
+        if (a.IsComplete()) { out[i] = true; continue; }     // also the reference's answer for a second call after success
+        const int r = csp.CheckResumable(a);
+        CSP::Lowered l;
+        csp.Lower(a, l);
+        dq_model* h = nullptr;
+        bool compiled = false;
+        for (const Seen& s : seen) if (s.csp == &csp && s.key == l.key) { h = s.h; break; }
+        if (!h) {
+            bool cache_used = false;
+            for (const Seen& s : seen) if (s.csp == &csp && s.h == csp.cache_.handle) cache_used = true;
+            if (csp.cache_.handle && csp.cache_.key == l.key) h = csp.cache_.handle;
+            else if (!cache_used) {
+                csp.cache_.Drop();
+                csp.cache_.handle = h = CSP::Compile(l, (int)csp.vars.size());
+                csp.cache_.key = l.key;
+                compiled = true;
+            } else {
+                h = CSP::Compile(l, (int)csp.vars.size());
+                call_handles.h.push_back(h);
+                compiled = true;
+            }
+            seen.push_back(Seen{&csp, l.key, h});
+        }
+        todo.push_back(i);
+        handles.push_back(h);
+        resumed.push_back(r);
+        fresh.push_back(compiled);
+        off.push_back(off.back() + csp.vars.size());
+    }
+    if (todo.empty()) return out;
+    const size_t m = todo.size();
+    std::vector<int32_t> outcome(m), first(std::max<size_t>(off.back(), 1));
+    std::vector<uint64_t> sols(m), nodes(m);
+    int64_t n_split = 0;
+    dq_tree_opts o{};
+    o.mode = DQ_MODE_FIRST;
+    o.part_count = 1;
+    const int rc = dq_solve_models(handles.data(), (int64_t)m, &o, outcome.data(), sols.data(), nodes.data(), first.data(),
+                                   &n_split, nullptr);
+    if (rc != DQ_OK) throw Error(rc, dq_last_error());
+    for (size_t k = 0; k < m; k++) {
+        const size_t i = todo[k];
+        const bool have = outcome[k] == DQ_SAT;
+        out[i] = csps[i]->FinishB200(*as[i], nodes[k], have, first.data() + off[k], resumed[k]);
+        if (reps) {
+            SolveReport& rep = (*reps)[i];
+            rep.tree.outcome = outcome[k];
+            rep.tree.n_solutions = sols[k];
+            rep.tree.n_nodes = nodes[k] - (uint64_t)resumed[k];
+            rep.tree.first_key = have ? 0 : UINT64_MAX;
+            rep.compiled_fresh = fresh[k] != 0;
+        }
+    }
+    return out;
 }
 
 }  // namespace b200

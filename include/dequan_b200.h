@@ -214,6 +214,18 @@ int dq_solve_tree(dq_model *m, const dq_tree_opts *opts,
 int dq_solve_tree_multi(dq_model *m, const dq_tree_opts *opts, int32_t n_devices, const int32_t *devices,
                         dq_tree_result *res, int32_t *first_solution);
 
+/* Many independent models in one call: per model, what dq_solve_tree(models[i], opts, ...) returns.  Small trees are
+ * searched one warp per model in one launch; a tree that outgrows a warp's node budget is solved by the split search
+ * afterwards (*n_split counts them).  solutions: first solutions concatenated in list order, model i's n_vars values
+ * starting at the sum of the earlier models' n_vars (InstVar::UNASSIGNED where none); NULL = not wanted.
+ * opts: mode FIRST or COUNT_ALL, engine AUTO or WARP, one partition, no split depth, no node budget.  A handle may
+ * appear more than once; every handle belongs to the calling thread and must not be bound to another device.
+ * stats (may be NULL): n_sat / n_unsat, total_nodes, kernel_ms = device time of the in-batch launches,
+ * kernel_launches including the split solves, h2d_bytes / d2h_bytes of the batch's own copies; n_budget is 0.      */
+int dq_solve_models(dq_model *const *models, int64_t n, const dq_tree_opts *opts, int32_t *outcome,
+                    uint64_t *n_solutions, uint64_t *n_nodes, int32_t *solutions, int64_t *n_split,
+                    dq_batch_stats *stats);
+
 /* FIRST-mode node accounting across partitions (multi-GPU): after dq_solve_tree, the number of
  * nodes (AssignVar calls, dequan.h:416-423) the reference's sequential search would have visited
  * up to and including the solution inside prefix `key`, restricted to the subtrees this
