@@ -38,6 +38,7 @@ class ConKind(IntEnum):  # include/dequan_b200.h dq_con_kind
     ALLDIFF = 2
     ORRANGE = 3
     TABLE = 4
+    FILTER = 5
 
 
 @dataclass
@@ -114,6 +115,29 @@ class TableConstraint:
 
     def text(self):
         return f"table {self.v0} {self.v1} {len(self.pairs)} " + " ".join(f"{a} {b}" for a, b in self.pairs)
+
+
+@dataclass
+class FilterConstraint:
+    """A user-defined binary `dequan::Constraint` that overrides AplyArcConsistency (dequan.h:145-147), tabulated the
+    way include/dequan.h's TabulateUserConstraint does it: `allow` = the (v0, v1) value pairs its Evaluate accepts;
+    `keep01` = the pairs (a, b) such that assigning v0 = a leaves b in v1's domain; `keep10` = the pairs (a, b) such that
+    assigning v1 = b leaves a in v0's domain.  Every pair is (value of v0, value of v1)."""
+    v0: int
+    v1: int
+    allow: List[tuple]
+    keep01: List[tuple]
+    keep10: List[tuple]
+
+    def lower(self):
+        flat = [self.v0, self.v1, len(self.allow), len(self.keep01), len(self.keep10)]
+        for pairs in (self.allow, self.keep01, self.keep10):
+            for a, b in pairs:
+                flat += [a, b]
+        return ConKind.FILTER, flat
+
+    def text(self):
+        raise NotImplementedError("the reference driver's .dqm format has no filtering user constraint")
 
 
 class dq_model_desc(C.Structure):  # include/dequan_b200.h

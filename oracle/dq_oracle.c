@@ -204,8 +204,15 @@ static void restore_step(search_t *s) {
 
 enum { EV_NA = 0, EV_PASSED = 1, EV_FAILED = 2 };                 /* Constraint::Eval, dequan.h:136-141 */
 
+/* (a, b) is one of the n value pairs at p (a FILTER's allow or keep list; repeats and foreign values are harmless) */
+static int has_pair(const int32_t *p, int n, int a, int b) {
+    for (int i = 0; i < n; i++) if (p[2 * i] == a && p[2 * i + 1] == b) return 1;
+    return 0;
+}
+
 /* OpConstraint::Evaluate dequan.h:593-630; EqualityConstraint 700-709; OrRange 844-854;
- * AllDifferent 902-914; TABLE = user constraint as in oracle/ref_driver.cpp TableConstraint */
+ * AllDifferent 902-914; TABLE = user constraint as in oracle/ref_driver.cpp TableConstraint; FILTER = a user
+ * constraint with its own filter, as tests/cpp/dropin_scenarios.cpp OrderedConstraint */
 static int evaluate(search_t *s, const con_t *k, int last) {
     const int32_t *d = k->data;
     switch (k->kind) {
@@ -241,6 +248,11 @@ static int evaluate(search_t *s, const con_t *k, int last) {
         for (int i = 2; i + 1 < k->n; i += 2) if (d[i] == a && d[i + 1] == b) return EV_PASSED;
         return EV_FAILED;
     }
+    case DQ_CON_FILTER: {
+        int a = s->inst[d[0]], b = s->inst[d[1]];
+        if (a == UNASSIGNED || b == UNASSIGNED) return EV_NA;
+        return has_pair(d + 5, d[2], a, b) ? EV_PASSED : EV_FAILED;
+    }
     }
     return EV_NA;
 }
@@ -261,7 +273,8 @@ static int op_filter(search_t *s, int vid, int oth, int op) {
 }
 
 /* AplyArcConsistency of each kind: Op dequan.h:631-694 (op reversal 681-690), Equality 710-743,
- * OrRange 855-894 (body compiled out), AllDifferent 915-939, TABLE = base-class default 147 */
+ * OrRange 855-894 (body compiled out), AllDifferent 915-939, TABLE = base-class default 147, FILTER = the user's
+ * override (dequan.h:145-147) */
 static int apply_arc(search_t *s, const con_t *k, int last) {
     const int32_t *d = k->data;
     switch (k->kind) {
@@ -302,6 +315,32 @@ static int apply_arc(search_t *s, const con_t *k, int last) {
             }
         }
         return 1;
+    }
+    case DQ_CON_FILTER: {
+        /* a user constraint's own AplyArcConsistency, tabulated (include/dequan.h TabulateUserConstraint): with one
+         * endpoint assigned, the other keeps the values its keep list pairs with the assigned value.  Values leave
+         * through Exclude, so the order of the rest is unchanged. */
+        s->applied++;
+        int a = s->inst[d[0]], b = s->inst[d[1]];
+        if ((a == UNASSIGNED) == (b == UNASSIGNED)) return 1;
+        const int x_is_v0 = a != UNASSIGNED, q = x_is_v0 ? d[1] : d[0];
+        const int32_t *keep = d + 5 + 2 * d[2] + (x_is_v0 ? 0 : 2 * d[3]);
+        const int n_keep = x_is_v0 ? d[3] : d[4];
+        ensure_saved(s, q);
+        dom_t *dm = &s->cur[q];
+        ivec vals = {0};                                  /* a snapshot: Exclude edits dm */
+        if (dm->type == DQ_DOM_VALUES) {
+            for (int i = 0; i < dm->vals.n; i++) iv_push(&vals, dm->vals.v[i]);
+        } else {
+            for (int r = 0; r < dm->vals.n; r += 2)
+                for (int w = dm->vals.v[r]; w < dm->vals.v[r + 1]; w++) iv_push(&vals, w);
+        }
+        for (int i = 0; i < vals.n; i++) {
+            const int w = vals.v[i];
+            if (!(x_is_v0 ? has_pair(keep, n_keep, a, w) : has_pair(keep, n_keep, w, b))) dom_exclude(dm, w);
+        }
+        free(vals.v);
+        return dm->vals.n != 0;
     }
     default: return 1;
     }
