@@ -47,6 +47,10 @@ class dq_batch_opts(C.Structure):
     _fields_ = [("node_budget", C.c_uint64), ("engine", C.c_int32), ("task_nodes", C.c_int32)]
 
 
+class dq_count_opts(C.Structure):
+    _fields_ = [("node_budget", C.c_uint64), ("solution_limit", C.c_uint64), ("engine", C.c_int32)]
+
+
 class dq_batch_stats(C.Structure):
     _fields_ = [("n_sat", C.c_uint64), ("n_unsat", C.c_uint64), ("n_budget", C.c_uint64), ("total_nodes", C.c_uint64),
                 ("kernel_ms", C.c_double), ("kernel_launches", C.c_uint64), ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64),
@@ -55,6 +59,7 @@ class dq_batch_stats(C.Structure):
 
 EXPORTS = ["dq_device_info", "dq_set_device", "dq_compile", "dq_free", "dq_model_info", "dq_model_order", "dq_model_table_bytes", "dq_solve_tree",
            "dq_solve_tree_multi", "dq_solve_models", "dq_tree_nodes_upto", "dq_enumerate_solutions", "dq_solve_batch_cells", "dq_solve_batch_cells_dev", "dq_solve_batch_graphs", "dq_solve_batch_graphs_dev",
+           "dq_count_batch_cells", "dq_count_batch_graphs",
            "dq_measure_int_peak", "dq_last_error", "dq_version", "dq_parse_sudoku_lines", "dq_parse_dimacs_col"]
 
 _lib = None
@@ -90,6 +95,10 @@ def lib():
                                         u8p, u64p, u8p, C.POINTER(dq_batch_stats)]
     L.dq_solve_batch_graphs_dev.argtypes = [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, u8p, C.c_int64, C.POINTER(dq_batch_opts),
                                             u8p, u64p, u8p, C.POINTER(dq_batch_stats)]
+    L.dq_count_batch_cells.argtypes = [vp, u8p, C.c_int64, C.c_int32, C.POINTER(dq_count_opts), u64p, u8p, u64p, u8p,
+                                       C.POINTER(dq_batch_stats)]
+    L.dq_count_batch_graphs.argtypes = [C.c_int32, C.c_int32, C.c_void_p, u8p, C.c_int64, C.POINTER(dq_count_opts),
+                                        u64p, u8p, u64p, u8p, C.POINTER(dq_batch_stats)]
     L.dq_measure_int_peak.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.dq_parse_sudoku_lines.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]
     L.dq_parse_dimacs_col.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_int32), C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]
@@ -154,6 +163,31 @@ class BatchResult:
     h2d_bytes: int
     d2h_bytes: int
     search_kernel_ms: float = 0.0
+
+
+@dataclass
+class CountResult:
+    """Per instance of a counting batch: `solutions` (uint64; min(total, limit) when limit > 0), `first` (the DFS-first
+    solution in the layout of the FIRST-mode batch, written whenever solutions >= 1), `nodes` and `status` (0 unsat,
+    1 sat, 2 budget, 3 bad given); then the batch totals."""
+    solutions: np.ndarray
+    first: np.ndarray
+    nodes: np.ndarray
+    status: np.ndarray
+    n_sat: int
+    n_unsat: int
+    n_budget: int
+    total_nodes: int
+    kernel_ms: float
+    launches: int
+    h2d_bytes: int
+    d2h_bytes: int
+    search_kernel_ms: float = 0.0
+
+
+def _count_result(sols, first, nodes, status, st) -> CountResult:
+    return CountResult(sols, first, nodes, status, st.n_sat, st.n_unsat, st.n_budget, st.total_nodes, st.kernel_ms,
+                       st.kernel_launches, st.h2d_bytes, st.d2h_bytes, st.search_kernel_ms)
 
 
 class Model:
@@ -260,6 +294,22 @@ class Model:
         return BatchResult(sol, nodes, status, st.n_sat, st.n_unsat, st.n_budget, st.total_nodes, st.kernel_ms,
                            st.kernel_launches, st.h2d_bytes, st.d2h_bytes)
 
+    def count_batch_cells(self, cells: np.ndarray, solution_limit: int = 0, node_budget: int = 0,
+                          engine: str = "auto") -> CountResult:
+        """dq_count_batch_cells: each instance's solutions, up to `solution_limit` (0 = all) and within `node_budget`
+        (0 = none).  cells: uint8[n, stride] host array (0 = keep template domain)."""
+        assert cells.dtype == np.uint8 and cells.ndim == 2 and cells.flags.c_contiguous
+        n, stride = cells.shape
+        sols = np.zeros(n, dtype=np.uint64)
+        first = np.zeros((n, stride), dtype=np.uint8)
+        nodes = np.zeros(n, dtype=np.uint64)
+        status = np.zeros(n, dtype=np.uint8)
+        o = dq_count_opts(node_budget, solution_limit, ENGINE[engine] if isinstance(engine, str) else int(engine))
+        st = dq_batch_stats()
+        _check(lib().dq_count_batch_cells(self._h, cells.ctypes.data, n, stride, C.byref(o), sols.ctypes.data,
+                                          first.ctypes.data, nodes.ctypes.data, status.ctypes.data, C.byref(st)))
+        return _count_result(sols, first, nodes, status, st)
+
     def solve_batch_cells_ptr(self, cells_ptr: int, n: int, stride: int, sol_ptr: int, nodes_ptr: int, status_ptr: int,
                               node_budget: int = 0, engine: str = "auto", device: bool = False, task_nodes: int = 0):
         """Raw-pointer form (pinned host buffers or, with device=True, HBM-resident buffers)."""
@@ -321,6 +371,25 @@ def solve_batch_graphs(n_vertices: int, k: int, edge_off: np.ndarray, edges: np.
                                        col.ctypes.data, nodes.ctypes.data, status.ctypes.data, C.byref(st)))
     return BatchResult(col, nodes, status, st.n_sat, st.n_unsat, st.n_budget, st.total_nodes, st.kernel_ms,
                        st.kernel_launches, st.h2d_bytes, st.d2h_bytes, st.search_kernel_ms)
+
+
+def count_batch_graphs(n_vertices: int, k: int, edge_off: np.ndarray, edges: np.ndarray, solution_limit: int = 0,
+                       node_budget: int = 0, engine: str = "auto") -> CountResult:
+    """dq_count_batch_graphs: each graph's k-colourings, up to `solution_limit` (0 = all) and within `node_budget`
+    (0 = none); `first` holds the DFS-first colouring (0xFF where none)."""
+    assert edge_off.dtype == np.int64 and edges.dtype == np.uint8
+    edges = np.ascontiguousarray(edges)
+    n = len(edge_off) - 1
+    sols = np.zeros(n, dtype=np.uint64)
+    col = np.zeros((n, n_vertices), dtype=np.uint8)
+    nodes = np.zeros(n, dtype=np.uint64)
+    status = np.zeros(n, dtype=np.uint8)
+    o = dq_count_opts(node_budget, solution_limit, ENGINE[engine] if isinstance(engine, str) else int(engine))
+    st = dq_batch_stats()
+    _check(lib().dq_count_batch_graphs(n_vertices, k, edge_off.ctypes.data, edges.ctypes.data, n, C.byref(o),
+                                       sols.ctypes.data, col.ctypes.data, nodes.ctypes.data, status.ctypes.data,
+                                       C.byref(st)))
+    return _count_result(sols, col, nodes, status, st)
 
 
 def solve_batch_graphs_ptr(n_vertices: int, k: int, edge_off: np.ndarray, edge_off_dev: int, edges_ptr: int, col_ptr: int,

@@ -228,6 +228,7 @@ struct dq_model {
     // batch scratch
     DevBuf<uint8_t> b_cells, b_solution, b_status;
     DevBuf<unsigned long long> b_nodes;
+    DevBuf<unsigned long long> b_nsol;          // dq_count_batch_cells: solutions per instance
     // sudoku lane engine scratch (task pool)
     DevBuf<SudokuDigest> s_digest;
     DevBuf<unsigned long long> s_ctrl;
@@ -1392,9 +1393,11 @@ int dq_solve_models(dq_model* const* models, int64_t n, const dq_tree_opts* opts
 static int run_batch_sudoku(dq_model* m, const uint8_t* cells_dev, int64_t n, int32_t stride, const dq_batch_opts* opts,
                             uint8_t* sol_dev, unsigned long long* nodes_dev, uint8_t* status_dev, dq_batch_stats* st);
 
+// nsol_dev non-null: the counting batch (k_count_batch_cells, engine WARP) with solution limit `limit`.
 static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int32_t stride, const dq_batch_opts* opts,
                            uint8_t* sol_dev, unsigned long long* nodes_dev, uint8_t* status_dev, dq_batch_stats* st,
-                           const int* idx_list = nullptr, bool timed = true) {
+                           const int* idx_list = nullptr, bool timed = true, unsigned long long* nsol_dev = nullptr,
+                           unsigned long long limit = 0) {
     if (m->cm.wide()) { g_err = "batches take template domains of at most 32 values"; return DQ_ERR_UNSUPPORTED; }
     if (!idx_list && m->cm.model_class == CLASS_SUDOKU9 && !(opts && opts->engine == DQ_ENGINE_WARP))
         return run_batch_sudoku(m, cells_dev, n, stride, opts, sol_dev, nodes_dev, status_dev, st);
@@ -1406,8 +1409,9 @@ static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int
     const TreeModelDev M = dev_model(m);
     const size_t smem = warp_state_bytes(nv, M.trail) * kWarpsPerCta;
     if (smem > 200 * 1024) { g_err = "model state exceeds shared memory"; return DQ_ERR_UNSUPPORTED; }
+    const auto kernel = with_features(m->cm, [&](auto hf, auto ht) { return nsol_dev ? k_count_batch_cells<hf, ht> : k_batch_cells<hf, ht>; });
     int occ = 0;
-    int rc = with_features(m->cm, [&](auto hf, auto ht) { return max_ctas_per_sm(k_batch_cells<hf, ht>, kWarpsPerCta * 32, smem, &occ); });
+    int rc = max_ctas_per_sm(kernel, kWarpsPerCta * 32, smem, &occ);
     if (rc != DQ_OK) return rc;
     if (occ < 1) { g_err = "kernel does not fit an SM"; return DQ_ERR_UNSUPPORTED; }
     unsigned long long* ctrl = m->d_ctrl.p;
@@ -1418,10 +1422,11 @@ static int run_batch_cells(dq_model* m, const uint8_t* cells_dev, int64_t n, int
     A.sizes = m->t_sizes; A.n_sizes = m->n_sizes; A.caller_order = m->cm.caller_order ? 1 : 0;
     A.budget = opts ? opts->node_budget : 0;
     A.cursor = ctrl; A.solution = sol_dev; A.nodes = nodes_dev; A.status = status_dev; A.totals = ctrl + 1;
+    A.limit = limit; A.n_solutions = nsol_dev;
     long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)occ * ctx->sm_count);
     if (ctas < 1) ctas = 1;
     if (timed) DQ_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-    with_features(m->cm, [&](auto hf, auto ht) { k_batch_cells<hf, ht><<<(int)ctas, kWarpsPerCta * 32, smem, ctx->stream>>>(M, A); });
+    kernel<<<(int)ctas, kWarpsPerCta * 32, smem, ctx->stream>>>(M, A);
     DQ_CUDA(cudaGetLastError());
     if (!timed) return DQ_OK;
     DQ_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -1555,12 +1560,13 @@ int dq_solve_batch_cells_dev(dq_model* m, const uint8_t* cells_dev, int64_t n, i
     return run_batch_cells(m, cells_dev, n, stride, opts, solution_dev, (unsigned long long*)nodes_dev, status_dev, stats);
 }
 
-int dq_solve_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t stride, const dq_batch_opts* opts,
-                         uint8_t* solution, uint64_t* nodes, uint8_t* status, dq_batch_stats* stats) {
-    if (!m || n < 0 || stride < m->cm.nv) { g_err = "bad argument"; return DQ_ERR_INVALID; }
-    if (stats) memset(stats, 0, sizeof *stats);
-    if (n == 0) return DQ_OK;
-    if (!cells || !solution || !nodes || !status) { g_err = "null buffer"; return DQ_ERR_INVALID; }
+}  // extern "C"
+
+// dq_solve_batch_cells and dq_count_batch_cells (n_solutions non-null) once their arguments are checked: the host
+// buffers around run_batch_cells.
+static int batch_cells_host(dq_model* m, const uint8_t* cells, int64_t n, int32_t stride, const dq_batch_opts* opts,
+                            uint8_t* solution, uint64_t* nodes, uint8_t* status, dq_batch_stats* stats,
+                            uint64_t* n_solutions = nullptr, unsigned long long limit = 0) {
     int rc = upload(m);
     if (rc != DQ_OK) return rc;
     DeviceCtx* ctx = m->ctx;
@@ -1574,15 +1580,52 @@ int dq_solve_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t s
     const bool pinned = cudaPointerGetAttributes(&pa, solution) == cudaSuccess && pa.type == cudaMemoryTypeHost;
     if (!pinned) cudaGetLastError();
     m->early_sol_host = pinned ? solution : nullptr; m->early_sol_done = false;
-    rc = run_batch_cells(m, m->b_cells.p, n, stride, opts, m->b_solution.p, m->b_nodes.p, m->b_status.p, stats);
+    if (n_solutions) DQ_CUDA(m->b_nsol.reserve(n));
+    rc = run_batch_cells(m, m->b_cells.p, n, stride, opts, m->b_solution.p, m->b_nodes.p, m->b_status.p, stats, nullptr, true,
+                         n_solutions ? m->b_nsol.p : nullptr, limit);
     m->early_sol_host = nullptr;
     if (rc != DQ_OK) { cudaStreamSynchronize(ctx->stream2); return rc; }     // (nothing may still be writing the caller's buffer)
     if (!m->early_sol_done) DQ_CUDA(cudaMemcpyAsync(solution, m->b_solution.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CUDA(cudaMemcpyAsync(nodes, m->b_nodes.p, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CUDA(cudaMemcpyAsync(status, m->b_status.p, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_solutions) DQ_CUDA(cudaMemcpyAsync(n_solutions, m->b_nsol.p, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (stats) { stats->h2d_bytes = bytes; stats->d2h_bytes = bytes + (size_t)n * 9; }
+    if (stats) { stats->h2d_bytes = bytes; stats->d2h_bytes = bytes + (size_t)n * (n_solutions ? 17 : 9); }
     return DQ_OK;
+}
+
+// The counting batches run on the generic warp engine only: engine AUTO or WARP.
+static int check_count_opts(const dq_count_opts* opts) {
+    const int engine = opts ? opts->engine : DQ_ENGINE_AUTO;
+    if (engine == DQ_ENGINE_LANE || engine == DQ_ENGINE_REG) {
+        g_err = "batch counting runs on the generic warp engine only: engine AUTO or WARP"; return DQ_ERR_UNSUPPORTED;
+    }
+    if (engine != DQ_ENGINE_AUTO && engine != DQ_ENGINE_WARP) { g_err = "bad engine"; return DQ_ERR_INVALID; }
+    return DQ_OK;
+}
+
+extern "C" {
+
+int dq_solve_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t stride, const dq_batch_opts* opts,
+                         uint8_t* solution, uint64_t* nodes, uint8_t* status, dq_batch_stats* stats) {
+    if (!m || n < 0 || stride < m->cm.nv) { g_err = "bad argument"; return DQ_ERR_INVALID; }
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (n == 0) return DQ_OK;
+    if (!cells || !solution || !nodes || !status) { g_err = "null buffer"; return DQ_ERR_INVALID; }
+    return batch_cells_host(m, cells, n, stride, opts, solution, nodes, status, stats);
+}
+
+int dq_count_batch_cells(dq_model* m, const uint8_t* cells, int64_t n, int32_t stride, const dq_count_opts* opts,
+                         uint64_t* n_solutions, uint8_t* solution, uint64_t* nodes, uint8_t* status, dq_batch_stats* stats) {
+    if (!m || n < 0 || stride < m->cm.nv) { g_err = "bad argument"; return DQ_ERR_INVALID; }
+    int rc = check_count_opts(opts);
+    if (rc != DQ_OK) return rc;
+    if (m->cm.wide()) { g_err = "batches take template domains of at most 32 values"; return DQ_ERR_UNSUPPORTED; }
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (n == 0) return DQ_OK;
+    if (!cells || !n_solutions || !solution || !nodes || !status) { g_err = "null buffer"; return DQ_ERR_INVALID; }
+    const dq_batch_opts o{opts ? opts->node_budget : 0, DQ_ENGINE_WARP, 0};
+    return batch_cells_host(m, cells, n, stride, &o, solution, nodes, status, stats, n_solutions, opts ? opts->solution_limit : 0);
 }
 
 }  // extern "C"
@@ -1593,6 +1636,7 @@ struct GraphBatchDev {
     const long long* off; const uint8_t* edges; long long edge_bytes;    // edge_bytes: 2 * total rounded up to 16, readable
     uint8_t* colours; unsigned long long* nodes; uint8_t* status;
     const uint8_t* host_edges;                                           // host copy of the lists, if the caller has one
+    unsigned long long* n_solutions = nullptr;                           // counting batch (warp engine): solutions per instance
 };
 
 // Lane-per-instance engine (dq_group_graphs.cuh): two passes of k_graphs_adjacency (overflow statistics, records),
@@ -1665,8 +1709,9 @@ static int run_graphs_lane(int nv, int k, const int64_t* edge_off, const GraphBa
     return DQ_OK;
 }
 
+// B.n_solutions non-null: the counting batch (k_count_batch_graphs, engine WARP) with solution limit `limit`.
 static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphBatchDev& B, int64_t n, const dq_batch_opts* opts,
-                            dq_batch_stats* stats) {
+                            dq_batch_stats* stats, unsigned long long limit = 0) {
     DeviceCtx* ctx = nullptr;
     DQ_CUDA(device_ctx(&ctx));
     cudaStream_t s = ctx->stream;
@@ -1707,6 +1752,7 @@ static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphB
         A.budget = opts ? opts->node_budget : 0; A.cursor = d_ctrl.p; A.colours = B.colours; A.nodes = B.nodes;
         A.status = B.status; A.totals = d_ctrl.p + 1;
         A.trail = nv * k + 32;
+        A.limit = limit; A.n_solutions = B.n_solutions;
         DQ_CUDA(cudaEventRecord(ctx->ev0, s));
         if (reg_engine) {
             RegGraphsArgs R;
@@ -1723,15 +1769,16 @@ static int run_batch_graphs(int nv, int k, const int64_t* edge_off, const GraphB
         } else {
             const size_t smem = warp_state_bytes(nv, A.trail) * kWarpsPerCta;
             if (smem > 200 * 1024) { g_err = "instance state exceeds shared memory"; return DQ_ERR_UNSUPPORTED; }
+            const auto kernel = B.n_solutions ? k_count_batch_graphs : k_batch_graphs;
             int occ = 0;
-            int rc = max_ctas_per_sm(k_batch_graphs, kWarpsPerCta * 32, smem, &occ);
+            int rc = max_ctas_per_sm(kernel, kWarpsPerCta * 32, smem, &occ);
             if (rc != DQ_OK) return rc;
             DQ_CUDA(d_ent_off.reserve((size_t)n * (nv + 1))); DQ_CUDA(d_ent.reserve(2 * (size_t)std::max<long long>(total, 1)));
             A.ent_off = d_ent_off.p; A.ent = d_ent.p;
             k_graphs_build<<<(unsigned)((n + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, kWarpsPerCta * graphs_build_warp_bytes(nv), s>>>(A);
             long long ctas = std::min<long long>((n + kWarpsPerCta - 1) / kWarpsPerCta, (long long)std::max(occ, 1) * sms);
             DQ_CUDA(cudaEventRecord(ctx->ev2, s));
-            k_batch_graphs<<<(unsigned)ctas, kWarpsPerCta * 32, smem, s>>>(A);
+            kernel<<<(unsigned)ctas, kWarpsPerCta * 32, smem, s>>>(A);
             launches = 2;
         }
         DQ_CUDA(cudaEventRecord(ctx->ev3, s));
@@ -1757,6 +1804,44 @@ static int check_edge_off(const int64_t* edge_off, int64_t n) {
     return DQ_OK;
 }
 
+static int check_edges(int nv, const uint8_t* edges, long long total) {
+    for (long long e = 0; e < total; e++) {
+        const uint8_t u = edges[2 * e], v = edges[2 * e + 1];
+        if (u >= nv || v >= nv) { g_err = "edge endpoint out of range"; return DQ_ERR_INVALID; }
+        if (u == v) { g_err = "edge with u == v"; return DQ_ERR_UNSUPPORTED; }
+    }
+    return DQ_OK;
+}
+
+// dq_solve_batch_graphs and dq_count_batch_graphs (n_solutions non-null) once their arguments are checked: the host
+// buffers around run_batch_graphs.
+static int batch_graphs_host(int32_t nv, int32_t k, const int64_t* edge_off, const uint8_t* edges, int64_t n,
+                             const dq_batch_opts* opts, uint8_t* colours, uint64_t* nodes, uint8_t* status,
+                             dq_batch_stats* stats, uint64_t* n_solutions = nullptr, unsigned long long limit = 0) {
+    const long long total = edge_off[n];
+    DeviceCtx* ctx = nullptr;
+    DQ_CUDA(device_ctx(&ctx));
+    cudaStream_t s = ctx->stream;
+    DevBuf<long long> d_off; DevBuf<uint8_t> d_edges, d_col, d_status; DevBuf<unsigned long long> d_nodes, d_nsol;
+    StreamDrain drain{s};
+    const long long edge_bytes = (2 * total + 15) & ~15ll;
+    DQ_CUDA(d_off.reserve(n + 1)); DQ_CUDA(d_edges.reserve(std::max<long long>(edge_bytes, 16))); DQ_CUDA(d_col.reserve((size_t)n * nv));
+    DQ_CUDA(d_status.reserve(n)); DQ_CUDA(d_nodes.reserve(n));
+    if (n_solutions) DQ_CUDA(d_nsol.reserve(n));
+    DQ_CUDA(cudaMemcpyAsync(d_off.p, edge_off, (n + 1) * sizeof(long long), cudaMemcpyHostToDevice, s));
+    if (total) DQ_CUDA(cudaMemcpyAsync(d_edges.p, edges, 2 * total, cudaMemcpyHostToDevice, s));
+    GraphBatchDev B{d_off.p, d_edges.p, edge_bytes, d_col.p, d_nodes.p, d_status.p, edges, d_nsol.p};
+    int rc = run_batch_graphs(nv, k, edge_off, B, n, opts, stats, limit);
+    if (rc != DQ_OK) return rc;
+    DQ_CUDA(cudaMemcpyAsync(colours, d_col.p, (size_t)n * nv, cudaMemcpyDeviceToHost, s));
+    DQ_CUDA(cudaMemcpyAsync(nodes, d_nodes.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    DQ_CUDA(cudaMemcpyAsync(status, d_status.p, (size_t)n, cudaMemcpyDeviceToHost, s));
+    if (n_solutions) DQ_CUDA(cudaMemcpyAsync(n_solutions, d_nsol.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    DQ_CUDA(cudaStreamSynchronize(s));
+    if (stats) { stats->h2d_bytes = (size_t)(n + 1) * 8 + 2 * (size_t)total; stats->d2h_bytes = (size_t)n * (nv + (n_solutions ? 17 : 9)); }
+    return DQ_OK;
+}
+
 extern "C" {
 
 int dq_solve_batch_graphs(int32_t nv, int32_t k, const int64_t* edge_off, const uint8_t* edges, int64_t n,
@@ -1773,31 +1858,31 @@ int dq_solve_batch_graphs(int32_t nv, int32_t k, const int64_t* edge_off, const 
     if (opts && opts->engine == DQ_ENGINE_LANE && k > 4) { g_err = "the lane engine serves k <= 4"; return DQ_ERR_UNSUPPORTED; }
     // the lane engine checks the lists on the device (k_graphs_adjacency); the others trust them: one pass on the host
     const int engine = opts ? opts->engine : DQ_ENGINE_AUTO;
-    if (!(k <= 4 && (engine == DQ_ENGINE_LANE || (engine == DQ_ENGINE_AUTO && n >= 4096))))
-        for (long long e = 0; e < total; e++) {
-            const uint8_t u = edges[2 * e], v = edges[2 * e + 1];
-            if (u >= nv || v >= nv) { g_err = "edge endpoint out of range"; return DQ_ERR_INVALID; }
-            if (u == v) { g_err = "edge with u == v"; return DQ_ERR_UNSUPPORTED; }
-        }
-    DeviceCtx* ctx = nullptr;
-    DQ_CUDA(device_ctx(&ctx));
-    cudaStream_t s = ctx->stream;
-    DevBuf<long long> d_off; DevBuf<uint8_t> d_edges, d_col, d_status; DevBuf<unsigned long long> d_nodes;
-    StreamDrain drain{s};
-    const long long edge_bytes = (2 * total + 15) & ~15ll;
-    DQ_CUDA(d_off.reserve(n + 1)); DQ_CUDA(d_edges.reserve(std::max<long long>(edge_bytes, 16))); DQ_CUDA(d_col.reserve((size_t)n * nv));
-    DQ_CUDA(d_status.reserve(n)); DQ_CUDA(d_nodes.reserve(n));
-    DQ_CUDA(cudaMemcpyAsync(d_off.p, edge_off, (n + 1) * sizeof(long long), cudaMemcpyHostToDevice, s));
-    if (total) DQ_CUDA(cudaMemcpyAsync(d_edges.p, edges, 2 * total, cudaMemcpyHostToDevice, s));
-    GraphBatchDev B{d_off.p, d_edges.p, edge_bytes, d_col.p, d_nodes.p, d_status.p, edges};
-    rc = run_batch_graphs(nv, k, edge_off, B, n, opts, stats);
+    if (!(k <= 4 && (engine == DQ_ENGINE_LANE || (engine == DQ_ENGINE_AUTO && n >= 4096)))) {
+        rc = check_edges(nv, edges, total);
+        if (rc != DQ_OK) return rc;
+    }
+    return batch_graphs_host(nv, k, edge_off, edges, n, opts, colours, nodes, status, stats);
+}
+
+int dq_count_batch_graphs(int32_t nv, int32_t k, const int64_t* edge_off, const uint8_t* edges, int64_t n,
+                          const dq_count_opts* opts, uint64_t* n_solutions, uint8_t* colours, uint64_t* nodes,
+                          uint8_t* status, dq_batch_stats* stats) {
+    if (nv < 1 || nv > kMaxGraphVertices || k < 1 || k > 32 || n < 0) { g_err = "bad argument"; return DQ_ERR_INVALID; }
+    int rc = check_count_opts(opts);
     if (rc != DQ_OK) return rc;
-    DQ_CUDA(cudaMemcpyAsync(colours, d_col.p, (size_t)n * nv, cudaMemcpyDeviceToHost, s));
-    DQ_CUDA(cudaMemcpyAsync(nodes, d_nodes.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-    DQ_CUDA(cudaMemcpyAsync(status, d_status.p, (size_t)n, cudaMemcpyDeviceToHost, s));
-    DQ_CUDA(cudaStreamSynchronize(s));
-    if (stats) { stats->h2d_bytes = (size_t)(n + 1) * 8 + 2 * (size_t)total; stats->d2h_bytes = (size_t)n * (nv + 9); }
-    return DQ_OK;
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (n == 0) return DQ_OK;
+    if (!edge_off || !n_solutions || !colours || !nodes || !status) { g_err = "null buffer"; return DQ_ERR_INVALID; }
+    rc = check_edge_off(edge_off, n);
+    if (rc != DQ_OK) return rc;
+    const long long total = edge_off[n];
+    if (total && !edges) { g_err = "null edge buffer"; return DQ_ERR_INVALID; }
+    rc = check_edges(nv, edges, total);              // (the warp engine trusts the lists)
+    if (rc != DQ_OK) return rc;
+    const dq_batch_opts o{opts ? opts->node_budget : 0, DQ_ENGINE_WARP, 0};
+    return batch_graphs_host(nv, k, edge_off, edges, n, &o, colours, nodes, status, stats, n_solutions,
+                             opts ? opts->solution_limit : 0);
 }
 
 int dq_solve_batch_graphs_dev(int32_t nv, int32_t k, const int64_t* edge_off, const int64_t* edge_off_dev, const uint8_t* edges_dev,

@@ -312,6 +312,9 @@ struct BatchCellsArgs {
     uint8_t* status;            // [n]
     unsigned long long* totals; // [0]=sat [1]=unsat [2]=budget [3]=nodes
     const int* idx_list;        // optional: the n instance ids to solve (null = 0..n-1)
+    // counting batches (k_count_batch_cells) only
+    unsigned long long limit = 0;               // solution limit per instance (0 = every solution)
+    unsigned long long* n_solutions = nullptr;  // [n]
 };
 
 struct NoFirst {
@@ -319,11 +322,27 @@ struct NoFirst {
     __device__ void solutions(const WarpState&, uint32_t, unsigned long long) const {}
 };
 
-template <bool HAS_F, bool HAS_TABLE>
-__global__ void __launch_bounds__(kWarpsPerCta * 32)
-k_batch_cells(TreeModelDev M, BatchCellsArgs A) {
-    extern __shared__ __align__(16) unsigned char smem[];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+// Counting batches: the DFS-first solution goes to the instance's output row when it is found (the count searches on
+// and changes val[]), as bytes: values[v][index] for cell batches, the value index itself (the colour) when values is
+// null.
+struct FirstBytes {
+    uint8_t* out;
+    const int32_t* values;
+    int nv, lane;
+    __device__ void operator()(const WarpState& S) const {
+        for (int i = lane; i < nv; i += 32) {
+            const int v = S.order[i], b = S.val[i];
+            out[v] = values ? (uint8_t)__ldg(values + v * 32 + b) : (uint8_t)b;
+        }
+    }
+    __device__ void solutions(const WarpState&, uint32_t, unsigned long long) const {}
+};
+
+// One warp per instance, in turn.  COUNT: count its solutions up to A.limit (warp_dfs's LIMITED path) and write the
+// DFS-first one; else its FIRST-mode solve.  (The kernels pass in their shared memory and lane: so the FIRST-mode
+// kernels compile to the same code as when this body was theirs.)
+template <bool HAS_F, bool HAS_TABLE, bool COUNT>
+__device__ __forceinline__ void batch_cells(TreeModelDev M, BatchCellsArgs A, unsigned char* smem, int lane, int wib) {
     const int nv = M.T.nv;
     const uint32_t lt = (1u << lane) - 1u;
     WarpState S = carve_warp_state(smem + (size_t)wib * warp_state_bytes(nv, M.trail), nv, M.trail);
@@ -369,10 +388,18 @@ k_batch_cells(TreeModelDev M, BatchCellsArgs A) {
         __syncwarp();
         DfsResult R;
         if (bad) { R.nodes = 0; R.sols = 0; R.outcome = 0; R.have_first = false; }
+        else if constexpr (COUNT)
+            R = warp_dfs<HAS_F, HAS_TABLE, true>(M.T, S, 0, true, A.budget, nullptr, 0ull, lane,
+                                                 FirstBytes{A.solution + (size_t)i * A.stride, A.values, nv, lane}, A.limit);
         else R = warp_dfs<HAS_F, HAS_TABLE>(M.T, S, 0, false, A.budget, nullptr, 0ull, lane, NoFirst());
         uint8_t* out = A.solution + (size_t)i * A.stride;
-        for (int v = lane; v < nv; v += 32)
-            out[v] = R.outcome == 1 ? (uint8_t)__ldg(A.values + v * 32 + S.val[S.pos[v]]) : (uint8_t)0;
+        if constexpr (COUNT) {
+            if (!R.sols) for (int v = lane; v < nv; v += 32) out[v] = 0;
+            if (lane == 0) A.n_solutions[i] = R.sols;
+        } else {
+            for (int v = lane; v < nv; v += 32)
+                out[v] = R.outcome == 1 ? (uint8_t)__ldg(A.values + v * 32 + S.val[S.pos[v]]) : (uint8_t)0;
+        }
         if (lane == 0) { A.nodes[i] = R.nodes; A.status[i] = bad ? (uint8_t)3 : (uint8_t)R.outcome; }
         t_nodes += R.nodes;
         t_sat += R.outcome == 1; t_unsat += R.outcome == 0; t_budget += R.outcome == 2;
@@ -382,6 +409,20 @@ k_batch_cells(TreeModelDev M, BatchCellsArgs A) {
         atomicAdd(A.totals + 0, t_sat); atomicAdd(A.totals + 1, t_unsat);
         atomicAdd(A.totals + 2, t_budget); atomicAdd(A.totals + 3, t_nodes);
     }
+}
+
+template <bool HAS_F, bool HAS_TABLE>
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+k_batch_cells(TreeModelDev M, BatchCellsArgs A) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    batch_cells<HAS_F, HAS_TABLE, false>(M, A, smem, threadIdx.x & 31, threadIdx.x >> 5);
+}
+
+template <bool HAS_F, bool HAS_TABLE>
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+k_count_batch_cells(TreeModelDev M, BatchCellsArgs A) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    batch_cells<HAS_F, HAS_TABLE, true>(M, A, smem, threadIdx.x & 31, threadIdx.x >> 5);
 }
 
 // ---- batch: one graph per instance (k-colouring) ------------------------------------------------
@@ -401,6 +442,9 @@ struct BatchGraphsArgs {
     uint8_t* status;
     unsigned long long* totals;
     int trail;
+    // counting batches (k_count_batch_graphs) only
+    unsigned long long limit = 0;               // solution limit per instance (0 = every solution)
+    unsigned long long* n_solutions = nullptr;  // [n]
 };
 
 // k_graphs_build's shared memory per warp: deg[nv + 1] and an nv x nv adjacency bit matrix
@@ -456,10 +500,9 @@ k_graphs_build(BatchGraphsArgs A) {
     }
 }
 
-__global__ void __launch_bounds__(kWarpsPerCta * 32)
-k_batch_graphs(BatchGraphsArgs A) {
-    extern __shared__ __align__(16) unsigned char smem[];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+// As batch_cells, with the instance's adjacency from k_graphs_build.
+template <bool COUNT>
+__device__ __forceinline__ void batch_graphs(BatchGraphsArgs A, unsigned char* smem, int lane, int wib) {
     const int nv = A.nv;
     WarpState S = carve_warp_state(smem + (size_t)wib * warp_state_bytes(nv, A.trail), nv, A.trail);
     const uint32_t full = A.k >= 32 ? FULL : ((1u << A.k) - 1u);
@@ -477,9 +520,18 @@ k_batch_graphs(BatchGraphsArgs A) {
         T.masks = nullptr;
         for (int v = lane; v < nv; v += 32) { S.D[v] = full; S.F[v] = 0; S.order[v] = (uint16_t)v; S.pos[v] = (uint16_t)v; }
         __syncwarp();
-        DfsResult R = warp_dfs<false, false>(T, S, 0, false, A.budget, nullptr, 0ull, lane, NoFirst());
+        DfsResult R;
+        if constexpr (COUNT)
+            R = warp_dfs<false, false, true>(T, S, 0, true, A.budget, nullptr, 0ull, lane,
+                                             FirstBytes{A.colours + (size_t)i * nv, nullptr, nv, lane}, A.limit);
+        else R = warp_dfs<false, false>(T, S, 0, false, A.budget, nullptr, 0ull, lane, NoFirst());
         uint8_t* out = A.colours + (size_t)i * nv;
-        for (int v = lane; v < nv; v += 32) out[v] = R.outcome == 1 ? S.val[v] : (uint8_t)0xFF;
+        if constexpr (COUNT) {
+            if (!R.sols) for (int v = lane; v < nv; v += 32) out[v] = 0xFF;
+            if (lane == 0) A.n_solutions[i] = R.sols;
+        } else {
+            for (int v = lane; v < nv; v += 32) out[v] = R.outcome == 1 ? S.val[v] : (uint8_t)0xFF;
+        }
         if (lane == 0) { A.nodes[i] = R.nodes; A.status[i] = (uint8_t)R.outcome; }
         t_nodes += R.nodes;
         t_sat += R.outcome == 1; t_unsat += R.outcome == 0; t_budget += R.outcome == 2;
@@ -489,6 +541,18 @@ k_batch_graphs(BatchGraphsArgs A) {
         atomicAdd(A.totals + 0, t_sat); atomicAdd(A.totals + 1, t_unsat);
         atomicAdd(A.totals + 2, t_budget); atomicAdd(A.totals + 3, t_nodes);
     }
+}
+
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+k_batch_graphs(BatchGraphsArgs A) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    batch_graphs<false>(A, smem, threadIdx.x & 31, threadIdx.x >> 5);
+}
+
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+k_count_batch_graphs(BatchGraphsArgs A) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    batch_graphs<true>(A, smem, threadIdx.x & 31, threadIdx.x >> 5);
 }
 
 // ---- many independent models (dq_solve_models): one warp owns one model's whole tree -----------------------------

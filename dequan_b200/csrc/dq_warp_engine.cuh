@@ -153,15 +153,25 @@ __device__ __forceinline__ bool fc_apply(const DevTablesT<W>& T, const WarpState
     return __any_sync(FULL, wiped);
 }
 
+// Bit index of the n-th (1-based) set bit of x, which has at least n.
+template <typename W>
+__device__ __forceinline__ int dq_nth_bit(W x, int n) {
+    for (; n > 1; --n) x &= x - 1;
+    return dq_ffs(x) - 1;
+}
+
 // Explicit-stack DFS from depth d0 (domains already reflect the d0 assignments above it).
 //   count_all : walk the whole subtree (solutions + nodes); else stop at the DFS-first solution.
 //   budget    : stop once more than `budget` nodes have been counted (0 = none), outcome DQ_BUDGET.
 //   abort_key / my_key : FIRST-mode prefix search — give up when another warp has recorded a solution
 //                in an earlier prefix (abort_key may be null).
-template <bool HAS_F, bool HAS_TABLE, typename W, class OnFirst>
+//   LIMITED (count_all only): the counting constraint passes the `limit`-th solution (0 = none), so the search stops
+//                there with outcome DQ_SAT; the node count stops at that value or at node budget + 1 also inside the
+//                last level, where the plain count adds the whole level before it tests the budget.
+template <bool HAS_F, bool HAS_TABLE, bool LIMITED = false, typename W, class OnFirst>
 __device__ DfsResult warp_dfs(const DevTablesT<W>& T, const WarpStateT<W>& S, int d0, bool count_all,
                               unsigned long long budget, const unsigned long long* abort_key,
-                              unsigned long long my_key, int lane, OnFirst on_first) {
+                              unsigned long long my_key, int lane, OnFirst on_first, unsigned long long limit = 0) {
     const int nv = T.nv;
     DfsResult R;
     R.nodes = 0; R.sols = 0; R.outcome = 0; R.have_first = false;
@@ -183,6 +193,32 @@ __device__ DfsResult warp_dfs(const DevTablesT<W>& T, const WarpStateT<W>& S, in
         if (d == nv - 1) {
             // last variable: each remaining value is a node; valid ones are solutions, no filtering left to do
             const W valid = HAS_F ? (c & ~S.F[x]) : c;
+            if (LIMITED) {
+                W reach = c;                              // the values of this level the search visits
+                if (limit && (unsigned long long)dq_popc(valid) >= limit - R.sols) {
+                    const int b = dq_nth_bit(valid, (int)(limit - R.sols));
+                    reach = c & ((W(2) << b) - W(1));     // ... up to the one that completes the limit-th solution
+                }
+                if (budget && R.nodes + dq_popc(reach) > budget) {
+                    const int b = dq_nth_bit(c, (int)(budget - R.nodes) + 1);
+                    reach = c & ((W(1) << b) - W(1));     // ... before node budget + 1
+                    R.outcome = 2;
+                }
+                const W got = valid & reach;
+                R.nodes = R.outcome == 2 ? budget + 1 : R.nodes + dq_popc(reach);
+                if (got) on_first.solutions(S, got, R.sols);
+                if (got && !R.have_first) {
+                    R.have_first = true;
+                    if (lane == 0) S.val[d] = (uint8_t)(dq_ffs(got) - 1);
+                    __syncwarp();
+                    on_first(S);
+                }
+                R.sols += dq_popc(got);
+                if (R.outcome == 2) break;
+                if (limit && R.sols == limit) { R.outcome = 1; break; }
+                c = 0;
+                continue;
+            }
             if (count_all) {
                 R.nodes += dq_popc(c);
                 if (budget && R.nodes > budget) { R.outcome = 2; break; }

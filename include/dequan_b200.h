@@ -279,6 +279,40 @@ int dq_solve_batch_graphs_dev(int32_t n_vertices, int32_t k, const int64_t *edge
                               const dq_batch_opts *opts, uint8_t *colours_dev, uint64_t *nodes_dev,
                               uint8_t *status_dev, dq_batch_stats *stats);
 
+/* ---- counting batches --------------------------------------------------------
+ * The instances of dq_solve_batch_cells / dq_solve_batch_graphs (same givens, status 3
+ * rows, search order), each searched to the end with a counting Constraint linked last to
+ * the last variable (SURVEY.md §8c) that passes, instead of failing, the solution_limit-th
+ * solution: ForwardCheckingStep returns true there.  The node budget is checked on every
+ * AssignVar before that constraint, as in the FIRST-mode batches.  Per instance:
+ *   n_solutions[i]  every solution (limit 0); min(total, limit) (limit > 0: == limit means
+ *                   "at least limit"); the solutions counted before the budget ran out;
+ *   nodes[i]        AssignVar calls up to and including the node the search stopped at
+ *                   (the whole tree, the one completing the limit-th solution, or budget + 1);
+ *   status[i]       DQ_SAT (>= 1 solution, tree exhausted or limit reached), DQ_UNSAT,
+ *                   DQ_BUDGET (budget ran out first, whatever was counted), 3 (bad given:
+ *                   0 nodes, 0 solutions);
+ *   solution[i] / colours[i]  the DFS-first solution whenever n_solutions[i] >= 1, in the
+ *                   layout of the FIRST-mode batch; otherwise 0 (cells) / 0xFF (graphs).
+ * With solution_limit 1, status, nodes and solution equal the FIRST-mode batch's.  The
+ * count runs on the generic warp engine: engine AUTO or WARP (LANE and REG are refused
+ * with DQ_ERR_UNSUPPORTED).  opts NULL = every solution, no budget, AUTO.  stats as for
+ * the FIRST-mode batches.  Host buffers.                                                    */
+typedef struct dq_count_opts {
+    uint64_t node_budget;    /* per instance, 0 = unlimited                         */
+    uint64_t solution_limit; /* per instance, 0 = count every solution              */
+    int32_t  engine;         /* dq_engine: AUTO or WARP                             */
+} dq_count_opts;
+
+int dq_count_batch_cells(dq_model *tmpl, const uint8_t *cells, int64_t n, int32_t stride,
+                         const dq_count_opts *opts, uint64_t *n_solutions, uint8_t *solution,
+                         uint64_t *nodes, uint8_t *status, dq_batch_stats *stats);
+
+int dq_count_batch_graphs(int32_t n_vertices, int32_t k, const int64_t *edge_off,
+                          const uint8_t *edges, int64_t n, const dq_count_opts *opts,
+                          uint64_t *n_solutions, uint8_t *colours, uint64_t *nodes,
+                          uint8_t *status, dq_batch_stats *stats);
+
 /* On-disk instance formats for the batch entry points (host-side parsing only).
  * Sudoku: one puzzle per line, 81 characters, '1'..'9' givens, '0' '.' '_' '*' blank; blank
  * lines and lines starting with '#' are skipped.  cells[i*81 + c] as dq_solve_batch_cells
