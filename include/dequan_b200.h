@@ -262,7 +262,8 @@ int dq_solve_batch_cells_dev(dq_model *tmpl, const uint8_t *cells_dev, int64_t n
 
 /* Batch of independent k-colouring instances (one graph per instance):
  * variables 0..n_vertices-1 = AddIntVar(0,k); one OpConstraint(u,v,NotEqual,0) per
- * edge.  edge_off[n+1] indexes edges[2*e], edges as (u,v) byte pairs (n_vertices<=256).
+ * edge.  edge_off[n+1] indexes edges[2*e], edges as (u,v) byte pairs (1 <= n_vertices <= 254;
+ * more is refused with DQ_ERR_INVALID, as by every graph entry point).
  * colours[i*n_vertices + v] = colour or 0xFF.                                     */
 int dq_solve_batch_graphs(int32_t n_vertices, int32_t k, const int64_t *edge_off,
                           const uint8_t *edges, int64_t n, const dq_batch_opts *opts,
